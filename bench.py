@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W                       headline: CDAE training samples/s, configs[2]
   python bench.py --workload {c1,c2,c4_sampled,c4_full,small} ...     the other configs of the metric
   python bench.py --impl reference [--workload ...]                   the reference-semantics CPU path (oracle port)
+  python bench.py ... --dump-outputs DIR                              also the outputs of the last timed step, as .npy
   N > 1: launched by torch.distributed.run, one rank per GPU (c3: data-parallel / item-sharded step; c4_*: users
   partitioned over ranks, no collective)
 
@@ -199,6 +200,35 @@ def profile_kernels(ctx, run_step, passes):
     prof = _lib.profile_read(ctx)
     _lib.check(lib.drb_ctx_profile_enable(ctx, 0))
     return {k: round(v[0] / passes, 5) for k, v in prof.items()}
+
+
+DUMP_BUDGET = 60_000_000           # bytes over all files of --dump-outputs: under 64 MB with room for the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes the device tensors a caller of the timed path receives after its last step as out_dir/<name>.npy, so that
+    two builds run with the same arguments can be compared output for output.  float64 stays float64, integers become
+    float64 (exact), other floats float32.  Smallest first, a tensor is written whole when it fits an equal share of the
+    budget still left, otherwise as a fixed sample of its rows, in row order: the first rows of numpy
+    default_rng(0).permutation(n_rows).  So the sample depends only on the shapes, and two tensors with the same number
+    of rows share the sampled rows of the smaller sample."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+
+    def np_dtype(t):
+        return np.float32 if t.dtype.is_floating_point and t.dtype != torch.float64 else np.float64
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel() * np.dtype(np_dtype(kv[1])).itemsize)
+    left = DUMP_BUDGET
+    for j, (name, t) in enumerate(items):
+        dt = np_dtype(t)
+        row = int(np.prod(t.shape[1:])) * np.dtype(dt).itemsize
+        share = left // (len(items) - j)
+        if t.dim() and t.shape[0] * row > share:
+            idx = np.sort(np.random.default_rng(0).permutation(t.shape[0])[:max(1, share // row)])
+            t = t[torch.as_tensor(idx, device=t.device)]
+        h = np.ascontiguousarray(t.detach().cpu().numpy(), dtype=dt)
+        np.save(os.path.join(out_dir, name + '.npy'), h)
+        left -= h.nbytes
 
 
 def base_line(cfg, metric, unit, value, world, K, W, ms_total, config, clocks, launches, scaling='weak'):
@@ -433,6 +463,8 @@ def run_cdae_native(args, cfg, D, arrays=None):
         step(s)
     ms_total, clock_info = timed_steps(D, step_counted, W, K, flush_l2=flush)
     launches = m.launch_count() - launches0[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'loss': loss_dev, 'W': m.W, 'W_': m.W_, 'V': m.V, 'b': m.b, 'b_': m.b_})
     loss_value = m.global_loss(loss_dev)                        # collective when parallel: every rank calls it
     ms_warm = None
     if flush:                                                   # also the steady-state, L2-warm number
@@ -483,7 +515,7 @@ def run_cdae_native(args, cfg, D, arrays=None):
         # (each is a full bench line of its own workload; `python bench.py --workload X` prints the same line alone)
         extras = {}
         sub = argparse.Namespace(**vars(args))
-        sub.steps, sub.warmup = max(args.steps, 20), max(args.warmup, 3)
+        sub.warmup, sub.dump_outputs = max(args.warmup, 3), None
         for name in ('c2', 'c4_sampled', 'c4_full', 'c1'):
             try:
                 extras[name] = RUNNERS[WORKLOADS[name]['model']][0](sub, dict(WORKLOADS[name]), D,
@@ -557,7 +589,7 @@ def run_dmf_native(args, cfg, D, arrays=None):
     import drecpy_b200 as drb
     from drecpy_b200.parallel import DataParallel
     ds, _ = make_data(cfg)
-    B, K, W = cfg['batch'], max(args.steps, 50), args.warmup
+    B, K, W = cfg['batch'], args.steps, args.warmup
     kw = {}
     if D.world > 1:
         kw = dict(data_parallel=DataParallel(D.dist))
@@ -586,6 +618,12 @@ def run_dmf_native(args, cfg, D, arrays=None):
         step(s)
     ms_total, clock_info = timed_steps(D, step_counted, W, K, flush_l2=flush)
     launches = m.launch_count() - l0[0]
+    if args.dump_outputs and D.rank == 0:
+        out = {'loss': loss}
+        for tower in ('user_nn', 'item_nn'):
+            for j, (kernel, bias) in enumerate(m.tower_weights(tower)):
+                out[f'{tower}_kernel_{j}'], out[f'{tower}_bias_{j}'] = kernel, bias
+        dump_outputs(args.dump_outputs, out)
     ms_warm, _ = timed_steps(D, step, 3, K, flush_l2=False)
     # end to end through fit()'s step (host sampler -> H2D -> step -> D2H loss): median over chunks of 50 steps
     chunks = []
@@ -690,7 +728,7 @@ def run_rank_sampled_native(args, cfg, D, arrays=None):
     d_c = torch.as_tensor(np.ascontiguousarray(padded), device=D.dev)
     d_n = torch.full((len(mine),), C, dtype=torch.int32, device=D.dev)
     out = m.rank_candidates_device(d_u, d_c, d_n, True)
-    K, W = max(3, min(args.steps, 10)), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     l0 = [0]
 
     def step(s):
@@ -699,6 +737,8 @@ def run_rank_sampled_native(args, cfg, D, arrays=None):
         m.rank_candidates_device(d_u, d_c, d_n, True, out=out)
     ms_total, clock_info = timed_steps(D, step, W, K)
     launches = m.launch_count() - l0[0]
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(('iids', 'scores', 'n_out'), out)))
     n_users_total = int(D.sum_over_ranks(len(mine)))
     kernels = profile_kernels(m._ctx, step, 2)
     # ---- e2e leg: the public call (host candidate generation, H2D, rank, D2H of the ranked lists, metrics); N=1 only
@@ -786,15 +826,18 @@ def run_topk_native(args, cfg, D, arrays=None):
     k = cfg['k']
     lo, hi = (m.n_users * D.rank) // D.world, (m.n_users * (D.rank + 1)) // D.world
     uids = torch.arange(lo, hi, dtype=torch.int32, device=D.dev)
-    K, W = max(3, min(args.steps, 20)), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     l0 = [0]
+    last = [None]
 
     def step(s):
         if s == W:
             l0[0] = m.launch_count()
-        m.topk_batch(uids, k, novelty=True, return_device=True)
+        last[0] = m.topk_batch(uids, k, novelty=True, return_device=True)
     ms_total, clock_info = timed_steps(D, step, W, K)
     launches = m.launch_count() - l0[0]
+    if args.dump_outputs and D.rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(('iids', 'scores', 'n_out'), last[0])))
     kernels = profile_kernels(m._ctx, step, 2)
     # ---- e2e: host uids -> H2D -> top-k -> D2H of the ranked lists (iids, scores, counts)
     h_u = np.arange(lo, hi, dtype=np.int32)
@@ -927,6 +970,8 @@ def run_c5_native(args, cfg, D, arrays=None):
         step(s)
     ms_total, clock_info = timed_steps(D, step_counted, W, K)
     launches = m.launch_count() - l0[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'loss': loss_dev, 'W': m.W, 'W_': m.W_, 'V': m.V, 'b': m.b, 'b_': m.b_})
     loss_value = m.global_loss(loss_dev)
     # e2e: host sampler -> pinned staging -> H2D -> step -> D2H loss, exactly fit()'s per-step body
     for _ in range(2):
@@ -1039,7 +1084,14 @@ def main():
     ap.add_argument('--c5-scale', type=float, default=1.0, help='c5: shrink users / items / interactions by this factor')
     ap.add_argument('--parallel', default='data', choices=['data', 'items'],
                     help='N>1: data = replicated weights + gradient all-reduce; items = item-sharded weights')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy, '
+                         'float32 / float64, at most 64 MB in all (larger outputs as a fixed sample of their rows)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the native path; the reference arm has none')
     cfg = dict(WORKLOADS[args.workload])
     if args.mask and 'mask' in cfg:
         cfg['mask'] = args.mask

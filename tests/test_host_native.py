@@ -1,11 +1,12 @@
 """Host-side pieces of libdrb (no GPU needed): library loads and exports every symbol of include/drb.h, the
 CPython RNG replay, PointSampler vs the live-reference goldens, corruption mask vs the oracle, and the
 ranking_evaluation protocol vs the live-reference goldens."""
-import ctypes as C
 import json
 import os
 import random
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -29,16 +30,30 @@ def test_library_exports_every_declared_symbol():
     assert lib.drb_version() == 100
 
 
+NO_DEVICE_CHILD = '''
+import ctypes as C
+import torch
+import drecpy_b200 as drb
+from drecpy_b200 import _lib
+assert not torch.cuda.is_available()
+h = _lib.vp()
+assert _lib.load().drb_ctx_create(0, C.byref(h)) == -2
+assert b'no CPU fallback' in _lib.load().drb_last_error()
+u, i, v = drb.synthetic_interactions(30, 40, 300)
+try:
+    drb.CDAE(hidden_factors=8, verbose=False, seed=1).fit(drb.InteractionData(u, i, v), epochs=1)
+except RuntimeError:
+    pass
+else:
+    raise AssertionError('fit() ran without a CUDA device')
+'''
+
+
 def test_no_cpu_fallback_without_device():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip('GPU present')
-    h = _lib.vp()
-    assert _lib.load().drb_ctx_create(0, C.byref(h)) == -2
-    assert b'no CPU fallback' in _lib.load().drb_last_error()
-    u, i, v = drb.synthetic_interactions(30, 40, 300)
-    with pytest.raises(RuntimeError):
-        drb.CDAE(hidden_factors=8, verbose=False, seed=1).fit(drb.InteractionData(u, i, v), epochs=1)
+    """In a child process that sees no CUDA device (so it also runs where a GPU is present)."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES='')
+    r = subprocess.run([sys.executable, '-c', NO_DEVICE_CHILD], cwd=ROOT, env=env, capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 @pytest.mark.parametrize('seed', [0, 10, 23, 2 ** 31 + 7, 2 ** 45 + 3])

@@ -1,5 +1,5 @@
-import sys, json, time
-sys.path.insert(0,'/root/repo')
+import os, sys, json, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import drecpy_b200 as drb
 from drecpy_b200 import _lib
