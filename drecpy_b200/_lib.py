@@ -131,6 +131,8 @@ SIGNATURES = {
     'drb_dmf_forward_pairs': (C.c_int, [vp, vp, vp, i32, vp]),
     'drb_dmf_rank_candidates': (C.c_int, [vp, vp, i32, vp, vp, i32, i32, vp, vp, vp]),
     'drb_dmf_invalidate_cache': (C.c_int, [vp]),
+    'drb_dmf_topk_scratch_bytes': (i64, [vp, i32]),
+    'drb_dmf_topk': (C.c_int, [vp, vp, i32, i32, i32, vp, i64, vp, vp, vp]),
     'drb_debug_cdae_capture_logits': (C.c_int, [vp, vp]),
     'drb_debug_split_tf32': (C.c_int, [vp, vp, i32, i32, i32, vp, vp, vp, vp, i32, i32]),
     'drb_debug_umma_gemm': (C.c_int, [vp, vp, vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, i32, i32, vp, i32]),

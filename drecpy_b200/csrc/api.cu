@@ -1585,6 +1585,170 @@ int drb_dmf_forward_pairs(drb_dmf* m, const int32_t* uids, const int32_t* iids, 
   return DRB_OK;
 }
 
+}  // extern "C"
+
+// Item tower once for every item of the catalog, chunk by chunk, into m->item_rep; the representations stay valid
+// until the next training step or drb_dmf_invalidate_cache (a single-user rank() does not recompute the whole catalog).
+static int dmf_refresh_item_rep(drb_dmf* m) {
+  if (m->item_rep_valid) return DRB_OK;
+  drb_ctx* ctx = m->ctx;
+  const int li = m->tw[1].n_layers - 1;
+  const int ldl = m->tw[1].ld[li];
+  int r;
+  for (int32_t o = 0; o < m->d.n_items; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, m->d.n_items - o);
+    if ((r = launch_iota(ctx, m->iids, c, o))) return r;
+    if ((r = dmf_tower_fwd(m, 1, m->iids, c))) return r;
+    DRB_CUDA_TRY(ctx, cudaMemcpyAsync(m->item_rep + (int64_t)o * ldl, m->tw[1].act[li], (size_t)c * ldl * 4,
+                                      cudaMemcpyDeviceToDevice, ctx->stream));
+  }
+  m->item_rep_valid = true;
+  return DRB_OK;
+}
+
+// Plan of a drb_dmf_topk call: list capacity, item ranges of the filter passes (swept from the highest item id down)
+// and the scratch layout.  DRB_TOPK_CAP / DRB_TOPK_NS / DRB_TOPK_GROWTH (read per call, as drb_cdae_topk reads them)
+// set the list capacity, the first range and the growth of the ranges from pass to pass.
+struct DmfTopkPlan {
+  int cap, growth, n_s, i_pad, words, w32;
+  int n_stages; int lo[12];          // pass s covers items [lo[s], s ? lo[s - 1] : n_items)
+  int64_t bytes;
+};
+static constexpr int kDmfTopkFallbackRows = 32;
+
+struct DmfTopkScratch {
+  float* irep_t; float* item_inv; uint64_t* lists; uint32_t* bits; int32_t* cnt; uint32_t* tau; float* tau_z;
+  int32_t* fb_count; int32_t* fb_users; int32_t* big_users; float* fb_rows;
+};
+
+static int64_t dmf_topk_carve(const drb_dmf* m, const DmfTopkPlan& P, void* base, DmfTopkScratch* s) {
+  const int64_t B = m->d.max_batch;
+  Carver c(base);
+  DmfTopkScratch t{};
+  t.irep_t = c.take<float>((int64_t)P.w32 * P.i_pad);
+  t.item_inv = c.take<float>(P.i_pad);
+  t.lists = c.take<uint64_t>(B * P.cap);
+  t.bits = c.take<uint32_t>(B * P.words);
+  t.cnt = c.take<int32_t>(B);
+  t.tau = c.take<uint32_t>(B);
+  t.tau_z = c.take<float>(B);
+  t.fb_count = c.take<int32_t>(64);        // [0] claimed fallback rows, [16 + pass] long lists of that pass's select
+  t.fb_users = c.take<int32_t>(kDmfTopkFallbackRows);
+  t.big_users = c.take<int32_t>(B);
+  t.fb_rows = c.take<float>((int64_t)kDmfTopkFallbackRows * P.i_pad);
+  if (s) *s = t;
+  return c.off;
+}
+
+static int dmf_topk_plan(const drb_dmf* m, int k, DmfTopkPlan* P) {
+  if (k < 1 || k > 2048) return drb_fail(DRB_E_INVALID, "drb_dmf_topk: k must be in [1, 2048] (got %d)", k);
+  const int cap_env = getenv("DRB_TOPK_CAP") ? atoi(getenv("DRB_TOPK_CAP")) : 0;
+  const int ns_env = getenv("DRB_TOPK_NS") ? atoi(getenv("DRB_TOPK_NS")) : 0;
+  const int g_env = getenv("DRB_TOPK_GROWTH") ? atoi(getenv("DRB_TOPK_GROWTH")) : 0;
+  const int I = m->d.n_items;
+  // a pass over (growth - 1) times the items seen so far adds about (growth - 1) k keys to the >= k kept ones; room
+  // for three times that (the capacity follows k up to the 8192 keys the select kernels take)
+  int cap = 2048;
+  while (cap < 8 * k && cap < 8192) cap <<= 1;
+  if (cap_env) cap = cap_env;
+  if (cap < 32 || cap > 8192 || (cap & (cap - 1)))
+    return drb_fail(DRB_E_INVALID, "drb_dmf_topk: DRB_TOPK_CAP must be a power of two in [32, 8192] (got %d)", cap);
+  P->cap = cap;
+  P->growth = g_env ? std::max(2, g_env) : ((3ll * 2 + 1) * k <= cap ? 3 : 2);
+  // first range: at least 4 k items (its k-th best is then a usable threshold), at most half the list
+  P->n_s = ns_env > 0 ? ns_env : (int)std::min<int64_t>(drb_round_up(std::max(1024, 4 * k), 128), cap / 2);
+  P->i_pad = (int)drb_round_up(I, 128);
+  P->words = P->i_pad / 32;
+  P->w32 = 32 * dmf_topk_nj(m->tw[0].width[m->tw[0].n_layers - 1]);
+  P->n_stages = 0;
+  int64_t b = P->n_s;
+  while (true) {                                   // b = items covered from the top after this pass
+    const int lo = b >= I ? 0 : (int)((I - b) / 128 * 128);
+    P->lo[P->n_stages++] = lo;
+    if (lo == 0) break;
+    int64_t nx = drb_round_up((int64_t)(I - lo) * P->growth, 128);
+    if (P->n_stages == 11 || nx + nx / 4 >= I) nx = I;     // no short last pass
+    b = nx;
+  }
+  P->bytes = dmf_topk_carve(m, *P, nullptr, nullptr);
+  return DRB_OK;
+}
+
+extern "C" {
+
+int64_t drb_dmf_topk_scratch_bytes(drb_dmf* m, int32_t k) {
+  if (!m) return drb_fail(DRB_E_INVALID, "drb_dmf_topk_scratch_bytes: NULL model"), -1;
+  DmfTopkPlan P;
+  if (dmf_topk_plan(m, k, &P)) return -1;
+  return P.bytes;
+}
+
+int drb_dmf_topk(drb_dmf* m, const int32_t* uids, int32_t n, int32_t k, int32_t novelty, void* scratch,
+                 int64_t scratch_bytes, int32_t* out_iid, float* out_score, int32_t* n_out) {
+  if (!m || !uids || !out_iid || !out_score || !n_out || !scratch || n < 0)
+    return drb_fail(DRB_E_INVALID, "drb_dmf_topk: bad argument");
+  DmfTopkPlan P;
+  int r;
+  if ((r = dmf_topk_plan(m, k, &P))) return r;
+  if (scratch_bytes < P.bytes)
+    return drb_fail(DRB_E_INVALID, "drb_dmf_topk: scratch of %lld bytes, k = %d needs %lld (drb_dmf_topk_scratch_bytes)",
+                    (long long)scratch_bytes, k, (long long)P.bytes);
+  if (n == 0) return DRB_OK;
+  drb_ctx* ctx = m->ctx;
+  DmfTopkScratch S;
+  dmf_topk_carve(m, P, scratch, &S);
+  const int lu = m->tw[0].n_layers - 1, li = m->tw[1].n_layers - 1;
+  const int I = m->d.n_items, width = m->tw[0].width[lu], ldl = m->tw[1].ld[li];
+  if ((r = dmf_refresh_item_rep(m))) return r;
+  if ((r = launch_dmf_topk_prep(ctx, m->item_rep, ldl, width, I, P.i_pad, S.irep_t, S.item_inv))) return r;
+  for (int32_t o = 0; o < n; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, n - o);
+    if ((r = dmf_tower_fwd(m, 0, uids + o, c))) return r;
+    int32_t* b_iid = out_iid + (int64_t)o * k;
+    float* b_score = out_score + (int64_t)o * k;
+    DRB_CUDA_TRY(ctx, cudaMemsetAsync(S.cnt, 0, (size_t)c * 4, ctx->stream));
+    DRB_CUDA_TRY(ctx, cudaMemsetAsync(S.tau, 0, (size_t)c * 4, ctx->stream));
+    DRB_CUDA_TRY(ctx, cudaMemsetAsync(S.fb_count, 0, 64 * 4, ctx->stream));
+    const uint32_t* bits = nullptr;
+    if (novelty) {     // the user's stored items (the rank path's `seen` rows) as a bitmap
+      DRB_CUDA_TRY(ctx, cudaMemsetAsync(S.bits, 0, (size_t)c * P.words * 4, ctx->stream));
+      BatchPrepArgs bp{};
+      bp.indptr = m->d.csr_indptr; bp.indices = m->d.csr_indices; bp.rows = uids + o;
+      bp.label_bits = S.bits; bp.words_per_row = P.words;
+      if ((r = launch_batch_prep(ctx, bp, c))) return r;
+      bits = S.bits;
+    }
+    DmfFilterArgs fa{};
+    fa.urep = m->tw[0].act[lu]; fa.ld_u = m->tw[0].ld[lu]; fa.n_users = c;
+    fa.irep_t = S.irep_t; fa.item_inv = S.item_inv; fa.i_pad = P.i_pad; fa.width = width;
+    fa.seen_bits = bits; fa.words_per_row = P.words; fa.tau_ord = S.tau;
+    fa.cnt = S.cnt; fa.lists = S.lists; fa.cap = P.cap;
+    for (int st = 0; st < P.n_stages; st++) {
+      const bool last = st == P.n_stages - 1;
+      fa.item_lo = P.lo[st]; fa.item_hi = st ? P.lo[st - 1] : I;
+      if ((r = launch_dmf_topk_filter(ctx, fa))) return r;
+      if ((r = launch_select_lists(ctx, S.lists, P.cap, S.cnt, S.tau, S.tau_z, k, last, last ? b_iid : nullptr,
+                                   last ? b_score : nullptr, last ? n_out + o : nullptr, S.fb_users, S.fb_count,
+                                   kDmfTopkFallbackRows, S.big_users, S.fb_count + 16 + st, c)))
+        return r;
+    }
+    // users whose list overflowed claimed fallback rows in the last select; almost always none, so one small read
+    // back per block decides whether the exact fallback is launched at all
+    int32_t claimed = 0;
+    DRB_CUDA_TRY(ctx, cudaMemcpyAsync(&claimed, S.fb_count, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    DRB_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (claimed == 0) continue;
+    TopkArgs t{};
+    t.ld = P.i_pad; t.n_items = I; t.uids = uids + o;
+    t.seen_indptr = m->d.csr_indptr; t.seen_indices = m->d.csr_indices; t.novelty = novelty; t.k = k;
+    t.out_iid = b_iid; t.out_score = b_score; t.n_out = n_out + o;
+    if ((r = launch_dmf_topk_fallback(ctx, t, c, m->tw[0].act[lu], m->tw[0].ld[lu], m->item_rep, ldl, width, S.fb_rows,
+                                      S.fb_users, S.fb_count, kDmfTopkFallbackRows)))
+      return r;
+  }
+  return DRB_OK;
+}
+
 int drb_dmf_rank_candidates(drb_dmf* m, const int32_t* uids, int32_t n, const int32_t* cand,
                             const int32_t* cand_count, int32_t max_cand, int32_t novelty, int32_t* out_iid,
                             float* out_score, int32_t* n_out) {
@@ -1593,19 +1757,8 @@ int drb_dmf_rank_candidates(drb_dmf* m, const int32_t* uids, int32_t n, const in
   drb_ctx* ctx = m->ctx;
   const int lu = m->tw[0].n_layers - 1, li = m->tw[1].n_layers - 1;
   const int ldl = m->tw[1].ld[li];
-  // item tower once for every item of the catalog, chunk by chunk; the representations stay valid until the next
-  // training step or drb_dmf_invalidate_cache (a single-user rank() no longer recomputes the whole catalog)
   int r;
-  if (!m->item_rep_valid) {
-    for (int32_t o = 0; o < m->d.n_items; o += m->d.max_batch) {
-      const int c = std::min(m->d.max_batch, m->d.n_items - o);
-      if ((r = launch_iota(ctx, m->iids, c, o))) return r;
-      if ((r = dmf_tower_fwd(m, 1, m->iids, c))) return r;
-      DRB_CUDA_TRY(ctx, cudaMemcpyAsync(m->item_rep + (int64_t)o * ldl, m->tw[1].act[li], (size_t)c * ldl * 4,
-                                        cudaMemcpyDeviceToDevice, ctx->stream));
-    }
-    m->item_rep_valid = true;
-  }
+  if ((r = dmf_refresh_item_rep(m))) return r;
   int64_t per = m->d.max_batch;
   if (max_cand > 4096) {
     per = std::min<int64_t>(per, rank_scratch_rows(m->rank_scratch_bytes, max_cand));

@@ -274,4 +274,25 @@ int launch_select_lists(drb_ctx* ctx, uint64_t* lists, int cap, int32_t* cnt, ui
 int launch_topk_fallback(drb_ctx* ctx, const TopkArgs& a, int n, const float* h, int ld_h, const float* table, int ld_t,
                          const float* bias, int width, float* rows, int32_t* fb_users, int32_t* fb_count, int fb_max);
 
+// ------------------------------------------------------------------ dmf_topk.cu (DMF full-catalog top-k, FFMA scores)
+// vectors are zero-padded to 32 * dmf_topk_nj(width) components (1, 2, 4, 8 or 16 groups of 32)
+int dmf_topk_nj(int width);
+// irep [n_items][ld_i] -> irep_t [32 nj][i_pad] (k-major, zero-padded) and item_inv [i_pad] = 1 / |t| as the rank path
+// forms it (0 past n_items); i_pad a multiple of 128
+int launch_dmf_topk_prep(drb_ctx* ctx, const float* irep, int ld_i, int width, int n_items, int i_pad, float* irep_t,
+                         float* item_inv);
+struct DmfFilterArgs {
+  const float* urep; int ld_u; int n_users;       // [n_users][ld_u] user tower output of the block
+  const float* irep_t; const float* item_inv; int i_pad;   // from launch_dmf_topk_prep
+  int width;
+  int item_lo, item_hi;                           // item range of this pass (item_lo % 128 == 0)
+  const uint32_t* seen_bits; int words_per_row;   // NULL (no novelty filter) or [n_users][words_per_row]
+  const uint32_t* tau_ord;                        // [n_users] a key is listed when its orderable score is > tau
+  int32_t* cnt; uint64_t* lists; int cap;         // [n_users], [n_users][cap] (cnt may exceed cap: overflow)
+};
+int launch_dmf_topk_filter(drb_ctx* ctx, const DmfFilterArgs& a);
+// users with n_out == -1 (claimed by the final select): exact scores into `rows` ([fb_max][a.ld]), then k_topk on them
+int launch_dmf_topk_fallback(drb_ctx* ctx, const TopkArgs& a, int n, const float* urep, int ld_u, const float* irep,
+                             int ld_i, int width, float* rows, int32_t* fb_users, int32_t* fb_count, int fb_max);
+
 #endif

@@ -7,22 +7,10 @@
 // Total order reproduced exactly: (score, iid) compared lexicographically, largest first, duplicates of the
 // same candidate collapsed (the reference builds a set).  Scores are ordered through a monotone float->uint map
 // packed with the item id into one 64-bit key, so ties on the score are broken by the larger item id.
-#include "kernels.h"
+#include "topk_common.cuh"
 
 namespace {
 
-__device__ __forceinline__ uint32_t f2ord(float f) {
-  const uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(uint32_t o) {
-  return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
 __device__ __forceinline__ bool row_contains(const int32_t* lo, int n, int32_t x) {
   int a = 0, b = n;
   while (a < b) {

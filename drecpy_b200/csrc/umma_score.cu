@@ -25,6 +25,7 @@
 // Orientation as in umma_loss.cu: MMA M = 128 items on the TMEM lanes, N = 256 users on the TMEM columns; an epilogue
 // warp holds 32 consecutive items of one user across its lanes, so one ballot says which of them pass.
 #include "umma_common.cuh"
+#include "topk_common.cuh"
 
 namespace {
 
@@ -77,31 +78,6 @@ __device__ __forceinline__ void sc_mbar_arrive_rank(uint32_t bar, uint32_t rank)
   // relaxed: the arrival only reports completed tcgen05.ld reads (see umma_loss.cu); a cluster-scope release would
   // first drain the warp's outstanding list stores
   asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(mapa_rank(bar, rank)) : "memory");
-}
-
-// Gives the queued keys of one epilogue warp their list slots (one atomicAdd per key, all issued before any is
-// consumed) and stores them.  A queue entry is the final 64-bit key (orderable score << 32 | item id) plus the user's
-// row in the block.  Not inlined: the filter loop has 16 call sites and must stay inside the instruction cache.
-__device__ __noinline__ void sc_flush_queue(const uint64_t* qk, const unsigned short* qu, int qn, int32_t* cnt,
-                                            uint64_t* lists, int cap) {
-  const int lane = threadIdx.x & 31;
-  __syncwarp();
-  uint64_t ent[SC_QCAP / 32];
-  int row[SC_QCAP / 32], pos[SC_QCAP / 32];
-#pragma unroll
-  for (int bq = 0; bq < SC_QCAP / 32; bq++) {
-    const int e = bq * 32 + lane;
-    pos[bq] = 0x7fffffff;
-    if (e < qn) {
-      ent[bq] = qk[e];
-      row[bq] = qu[e];
-      pos[bq] = atomicAdd(cnt + row[bq], 1);
-    }
-  }
-#pragma unroll
-  for (int bq = 0; bq < SC_QCAP / 32; bq++)
-    if (pos[bq] < cap) lists[(int64_t)row[bq] * cap + pos[bq]] = ent[bq];
-  __syncwarp();
 }
 
 // FILTER = false: first slice, every unseen item is listed (one warp-aggregated atomicAdd per (warp, user) reserves the
@@ -284,7 +260,7 @@ k_umma_score_filter(const __grid_constant__ CUtensorMap map_a_hi, const __grid_c
     if (FILTER) prefetch_users(unit0, 0);
     int qn = 0;                                    // entries in the queue (warp-uniform); it lives across tiles and is
     auto flush_queue = [&]() {                     // flushed when the next row of keys would not fit, and at the end
-      sc_flush_queue(my_q, my_qu, qn, p.cnt, p.lists, p.cap);
+      flush_key_queue<SC_QCAP>(my_q, my_qu, qn, p.cnt, p.lists, p.cap);
       qn = 0;
     };
     int tl = 0;

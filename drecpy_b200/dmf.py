@@ -287,24 +287,83 @@ class DMF(DeepRecommenderABC):
         if uid is None or iid is None: return None
         return self._rescale_value(self.forward_pairs([uid], [iid])[0])
 
+    def _sync_item_cache(self):
+        # the library caches the item tower of the whole catalog between steps; in-place writes to the arena from
+        # Python (weight injection, _revert_weights) bump the tensor version -> tell it
+        if getattr(self, '_params_version', None) != self._params._version:
+            _lib.check(_lib.load().drb_dmf_invalidate_cache(self._native))
+            self._params_version = self._params._version
+
+    def _rank_device(self, d_u, d_c, d_n, novelty):
+        """drb_dmf_rank_candidates on device arrays: (iids, un-rescaled scores, n_out) as device tensors."""
+        torch = self._torch
+        n, max_c = d_c.shape
+        self._sync_item_cache()
+        o_i = torch.empty((n, max_c), dtype=torch.int32, device=self._dev)
+        o_s = torch.empty((n, max_c), dtype=torch.float32, device=self._dev)
+        o_n = torch.empty(n, dtype=torch.int32, device=self._dev)
+        _lib.check(_lib.load().drb_dmf_rank_candidates(self._native, _lib.t_ptr(d_u), n, _lib.t_ptr(d_c),
+                                                       _lib.t_ptr(d_n), max_c, int(bool(novelty)),
+                                                       _lib.t_ptr(o_i), _lib.t_ptr(o_s), _lib.t_ptr(o_n)))
+        return o_i, o_s, o_n
+
     def _rank_batch(self, uids, cand, cand_count, novelty):
         torch = self._torch
         with self._lock:
-            n, max_c = cand.shape
-            # the library caches the item tower of the whole catalog between steps; in-place writes to the arena
-            # from Python (weight injection, _revert_weights) bump the tensor version -> tell it
-            if getattr(self, '_params_version', None) != self._params._version:
-                _lib.check(_lib.load().drb_dmf_invalidate_cache(self._native))
-                self._params_version = self._params._version
             d_u = torch.as_tensor(np.ascontiguousarray(uids, np.int32), device=self._dev)
             d_c = torch.as_tensor(np.ascontiguousarray(cand, np.int32), device=self._dev)
             d_n = torch.as_tensor(np.ascontiguousarray(cand_count, np.int32), device=self._dev)
-            o_i = torch.empty((n, max_c), dtype=torch.int32, device=self._dev)
-            o_s = torch.empty((n, max_c), dtype=torch.float32, device=self._dev)
-            o_n = torch.empty(n, dtype=torch.int32, device=self._dev)
-            _lib.check(_lib.load().drb_dmf_rank_candidates(self._native, _lib.t_ptr(d_u), n, _lib.t_ptr(d_c),
-                                                           _lib.t_ptr(d_n), max_c, int(bool(novelty)),
-                                                           _lib.t_ptr(o_i), _lib.t_ptr(o_s), _lib.t_ptr(o_n)))
+            o_i, o_s, o_n = self._rank_device(d_u, d_c, d_n, novelty)
             # rank() reports rescaled predictions (recommender_abc.py:460 calls _predict -> _rescale_value)
             scores = self._rescale_value(o_s.cpu().numpy())
             return o_i.cpu().numpy(), scores, o_n.cpu().numpy()
+
+    def topk_batch(self, uids, k, novelty=True, return_device=False):
+        """Full-catalog top-k for many users: (iids [n, k], scores [n, k], n_out [n]).  Row r is what _rank_batch
+        returns for uids[r] over range(n_items), truncated to k: the same item ids, and scores computed bit for bit
+        as the rank path computes them (drb_dmf_topk), rescaled as rank() reports them.  1 <= k <= 2048.
+        return_device=True: device tensors (scores rescaled on the device)."""
+        torch = self._torch
+        lib = _lib.load()
+        k = int(k)
+        with self._lock:
+            self._sync_item_cache()
+            nb = lib.drb_dmf_topk_scratch_bytes(self._native, k)
+            if nb < 0:
+                msg = lib.drb_last_error()
+                raise RuntimeError(f'libdrb error: {msg.decode() if msg else ""}')
+            scratch = getattr(self, '_topk_scratch', None)
+            if scratch is None or scratch.numel() < nb:    # allocated once, grown when a larger k needs more
+                scratch = self._topk_scratch = torch.empty(nb, dtype=torch.uint8, device=self._dev)
+            d_u = uids if torch.is_tensor(uids) else torch.as_tensor(np.ascontiguousarray(uids, np.int32), device=self._dev)
+            n = d_u.numel()
+            o_i = torch.empty((n, k), dtype=torch.int32, device=self._dev)
+            o_s = torch.empty((n, k), dtype=torch.float32, device=self._dev)
+            o_n = torch.empty(n, dtype=torch.int32, device=self._dev)
+            _lib.check(lib.drb_dmf_topk(self._native, _lib.t_ptr(d_u), n, k, int(bool(novelty)), _lib.t_ptr(scratch),
+                                        scratch.numel(), _lib.t_ptr(o_i), _lib.t_ptr(o_s), _lib.t_ptr(o_n)))
+            if n and int(o_n.min()) < 0:
+                # more candidate lists of one block overflowed than the device-side fallback has rows for: those
+                # users go through the rank path over the whole catalog, a few at a time (n x n_items candidates)
+                bad = torch.nonzero(o_n < 0).flatten()
+                cat = torch.arange(self.n_items, dtype=torch.int32, device=self._dev)
+                for o in range(0, bad.numel(), 256):
+                    rows = bad[o:o + 256]
+                    c = rows.numel()
+                    r_i, r_s, r_n = self._rank_device(d_u[rows].contiguous(), cat.expand(c, -1).contiguous(),
+                                                      torch.full((c,), self.n_items, dtype=torch.int32,
+                                                                 device=self._dev), novelty)
+                    o_i[rows], o_s[rows], o_n[rows] = r_i[:, :k], r_s[:, :k], torch.clamp(r_n, max=k)
+            if return_device:
+                return o_i, self._rescale_value(o_s), o_n
+            return o_i.cpu().numpy(), self._rescale_value(o_s.cpu().numpy()), o_n.cpu().numpy()
+
+    def _recommend(self, uid, n, novelty, threshold):
+        if n <= 2048:
+            o_i, o_s, o_n = self.topk_batch(np.array([uid], np.int32), int(n), novelty)
+            ranked = [(o_s[0, j], int(o_i[0, j])) for j in range(int(o_n[0]))]
+        else:
+            ranked = self._rank(uid, range(self.n_items), n, novelty)
+        if threshold is None:
+            return ranked
+        return [x for x in ranked if x[0] >= threshold]

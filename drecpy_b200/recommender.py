@@ -244,6 +244,42 @@ class DeepRecommenderABC(ABC):
             return ranked_items
         return list(filter(lambda x: x[0] >= threshold, ranked_items))
 
+    def recommend_batch(self, user_ids, n=10, novelty=True, interaction_threshold=None, chunk=8192):
+        """Batched recommend() over raw user ids: (items [U, n] raw ids, scores [U, n], counts [U]); row r holds what
+        recommend(user_ids[r], n, novelty, interaction_threshold) returns, counts[r] entries of it.  Padding: -1 for
+        integer raw item ids (None otherwise) and NaN scores.  1 <= n <= 2048; users go to the model's full-catalog
+        top-k (topk_batch) `chunk` at a time."""
+        assert self.fitted is True, 'The model requires to be fitted before being able to make predictions.'
+        n = int(n)
+        if not 1 <= n <= 2048:
+            raise ValueError(f'recommend_batch: n must be in [1, 2048] (got {n}); use recommend() for longer lists')
+        data = self._data
+        user_ids = np.asarray(user_ids)
+        uids = np.asarray(data.users_to_uids(user_ids)).astype(np.int32) if len(user_ids) else np.zeros(0, np.int32)
+        unknown = np.flatnonzero(uids < 0)
+        if len(unknown):
+            raise AssertionError(f'User {user_ids[unknown[0]]} was not found.')
+        raw = data.raw_items
+        U = len(uids)
+        int_ids = np.issubdtype(raw.dtype, np.integer)
+        items = np.full((U, n), -1, np.int64) if int_ids else np.full((U, n), None, object)
+        scores, counts = None, np.zeros(U, np.int64)
+        for o in range(0, U, chunk):
+            oi, os_, on = self.topk_batch(uids[o:o + chunk], n, novelty)
+            on = np.asarray(on, np.int64)
+            if scores is None:
+                scores = np.full((U, n), np.nan, os_.dtype)
+            valid = np.arange(n)[None, :] < on[:, None]
+            if interaction_threshold is not None:      # scores are descending: the threshold keeps a prefix
+                valid &= os_ >= interaction_threshold
+                on = valid.sum(axis=1)
+            items[o:o + chunk] = np.where(valid, raw[np.where(valid, oi, 0)], items[o:o + chunk])
+            scores[o:o + chunk] = np.where(valid, os_, scores[o:o + chunk])
+            counts[o:o + chunk] = on
+        if scores is None:
+            scores = np.full((U, n), np.nan, np.float32)
+        return items, scores, counts
+
     def rank(self, user_id, item_ids, novelty=True, skip_invalid_items=True, **kwds):
         assert self.fitted is True, 'The model requires to be fitted before being able to make predictions.'
         assert self._data.user_to_uid(user_id) is not None, f'User {user_id} was not found.'
@@ -351,7 +387,8 @@ class DeepRecommenderABC(ABC):
     # ------------------------------------------------------------------ persistence (recommender_abc.py:503-524)
     _TRANSIENT = ('_native', '_ctx', '_torch', '_workspace', '_slots', '_loss_host', '_loss_dev', '_stream', '_lock',
                   '_mask_rng', '_mask_stream', '_keep_dev', '_sampler', '_dp', '_dp_dev', '_dp_gather', '_label_count', '_dz1', '_h_buf', '_keepalive', '_next', '_pool',
-                  '_d_indptr', '_d_indices', '_d_seen_indptr', '_d_seen_indices', '_dev_sparse', '_logger', '_dev')
+                  '_d_indptr', '_d_indices', '_d_seen_indptr', '_d_seen_indices', '_dev_sparse', '_logger', '_dev',
+                  '_topk_scratch')
 
     def __getstate__(self):
         """joblib/pickle: device arenas go to host tensors, native handles are dropped and rebuilt on load."""

@@ -350,6 +350,15 @@ int drb_dmf_rank_candidates(drb_dmf* m, const int32_t* uids, int32_t n, const in
 /* drb_dmf_rank_candidates keeps the item tower's output for the whole catalog until the next drb_dmf_step; a caller
  * that writes the parameter arena itself (weight injection, _revert_weights: recommender_abc.py:346-352) says so. */
 int drb_dmf_invalidate_cache(drb_dmf* m);
+/* replaces: recommender_abc.py:391-419 (recommend -> _recommend = _rank over range(n_items)) -> :454-461 (DMF: one
+ * _predict per candidate, dmf.py:101-106, then nlargest), for n users at once.  uids: device [n]; out_iid / out_score
+ * [n][k], n_out [n] (device).  Row u == drb_dmf_rank_candidates(uids[u], whole catalog) truncated to k, ids and fp32
+ * scores bit for bit; n_out[u] == -1: list overflow beyond the device fallback, re-run the user through the rank path.
+ * scratch: caller-owned device memory of drb_dmf_topk_scratch_bytes(m, k) bytes (-1: bad argument, see
+ * drb_last_error).  1 <= k <= 2048.  Shares the item-tower cache of drb_dmf_rank_candidates. */
+int64_t drb_dmf_topk_scratch_bytes(drb_dmf* m, int32_t k);
+int drb_dmf_topk(drb_dmf* m, const int32_t* uids, int32_t n, int32_t k, int32_t novelty, void* scratch,
+                 int64_t scratch_bytes, int32_t* out_iid, float* out_score, int32_t* n_out);
 
 /* ------------------------------------------------------------------ kernel-level test hooks (tests/ only)
  * The tcgen05 GEMM building blocks of the CDAE step, exposed so that tests can check them in isolation against
