@@ -143,6 +143,8 @@ SIGNATURES = {
     'drb_leave_k_out': (C.c_int, [i64, vp, i64, f64, i32, i64, i64, i32, vp]),
     'drb_eval_lookup': (C.c_int, [i64, vp, vp, vp, vp, vp, vp, vp, f64, i32, vp]),
     'drb_eval_metrics': (C.c_int, [i64, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp, vp, vp]),
+    'drb_eval_topk_metrics': (C.c_int, [vp, i32, vp, vp, i32, vp, i32, f64, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32,
+                                        vp, vp, vp, vp]),
 }
 
 _lib = None

@@ -318,11 +318,12 @@ class DMF(DeepRecommenderABC):
             scores = self._rescale_value(o_s.cpu().numpy())
             return o_i.cpu().numpy(), scores, o_n.cpu().numpy()
 
-    def topk_batch(self, uids, k, novelty=True, return_device=False):
+    def topk_batch(self, uids, k, novelty=True, return_device=False, rescale=True):
         """Full-catalog top-k for many users: (iids [n, k], scores [n, k], n_out [n]).  Row r is what _rank_batch
         returns for uids[r] over range(n_items), truncated to k: the same item ids, and scores computed bit for bit
         as the rank path computes them (drb_dmf_topk), rescaled as rank() reports them.  1 <= k <= 2048.
-        return_device=True: device tensors (scores rescaled on the device)."""
+        return_device=True: device tensors (scores rescaled on the device).  rescale=False: the float32 p = max(1e-6,
+        cosine) of the rank path, not rescaled."""
         torch = self._torch
         lib = _lib.load()
         k = int(k)
@@ -355,8 +356,15 @@ class DMF(DeepRecommenderABC):
                                                                  device=self._dev), novelty)
                     o_i[rows], o_s[rows], o_n[rows] = r_i[:, :k], r_s[:, :k], torch.clamp(r_n, max=k)
             if return_device:
-                return o_i, self._rescale_value(o_s), o_n
-            return o_i.cpu().numpy(), self._rescale_value(o_s.cpu().numpy()), o_n.cpu().numpy()
+                return o_i, self._rescale_value(o_s) if rescale else o_s, o_n
+            h_s = o_s.cpu().numpy()
+            return o_i.cpu().numpy(), self._rescale_value(h_s) if rescale else h_s, o_n.cpu().numpy()
+
+    def _topk_device_scores(self, uids, k, novelty):
+        return self.topk_batch(uids, k, novelty, return_device=True, rescale=False)
+
+    def _reported_scores(self, scores):
+        return self._rescale_value(scores)
 
     def _recommend(self, uid, n, novelty, threshold):
         if n <= 2048:

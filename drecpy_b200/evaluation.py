@@ -6,10 +6,15 @@ DRecPy/Evaluation/Metrics/ranking.py (DCG :20-56, NDCG :59-91, HitRatio :94-114,
 What changes: the per-user candidate generation runs in libdrb's host C++ (drb_eval_candidates) and all users
 are scored in one batched GPU call (model.rank_batch) instead of 4 Python threads calling model.rank per user.
 Models without rank_batch (any object with .rank) and non-integer raw ids go through the same protocol in Python.
+
+recommendation_evaluation (DRecPy/Evaluation/Processes/recommendation_evaluation.py:18-192, restated: see its
+docstring) evaluates the full-catalog top-k of every test user; for CDAE / DMF the lists stay on the device and
+drb_eval_topk_metrics reduces them to per-user DCG / ideal DCG / hit counts there.
 """
 import math
 import os
 import random
+import time
 
 import numpy as np
 import pandas as pd
@@ -235,27 +240,61 @@ def _fast_evaluation(model, data, users, t_indptr, t_order, thr, n_pos, n_neg, g
             _lib.np_ptr(c_flat_c), _lib.np_ptr(np.ascontiguousarray(p_off[:-1])), _lib.np_ptr(np.ascontiguousarray(p_off[1:])),
             _lib.np_ptr(p_flat_c), _lib.np_ptr(ks_c), len(ks), nthr, _lib.np_ptr(dcg), _lib.np_ptr(idcg),
             _lib.np_ptr(hits_all)))
-        for m in metrics:
-            for j, k_ in enumerate(ks):
-                n_rec = np.minimum(n_out, k_)
-                if type(m) is NDCG:
-                    cur, best = dcg[:, j], idcg[:, j]
-                    good = best != 0                                # ZeroDivisionError -> metric skipped for the user
-                    vals = (cur[good] / best[good]).tolist()
-                else:
-                    hits = hits_all[:, j]
-                    if type(m) is Precision:
-                        good = n_rec > 0
-                        vals = (hits[good] / n_rec[good]).tolist()
-                    else:                                           # HitRatio, Recall: / number of positives
-                        good = p_lens > 0
-                        vals = (hits[good] / p_lens[good]).tolist()
-                acc = 0
-                for v in vals:                                      # same left-to-right float additions as the loop
-                    acc += v
-                metric_sums[(m.name, k_)] = [acc, len(vals)]
+        n_rec = np.minimum(np.asarray(n_out)[:, None], np.asarray(ks)[None, :])
+        _metric_sums_from_user_values(metric_sums, metrics, ks, dcg, idcg, hits_all, n_rec, p_lens, p_lens)
+    return _metric_results(metric_sums)
+
+
+def _metric_sums_from_user_values(metric_sums, metrics, ks, dcg, idcg, hits_all, n_rec, n_pos, n_pos_distinct):
+    """The built-in metrics of every evaluated user from its per-cut-off sums ([n_users, len(ks)] arrays: DCG, ideal DCG,
+    hits among the first n_rec recommendations), added left to right in user order into metric_sums -- the same float
+    operations in the same order as the per-user metric calls.  n_pos: length of the sampled positives list (Recall);
+    n_pos_distinct: its distinct items (HitRatio divides by the size of a set).  A user whose metric would divide by
+    zero is skipped for that (metric, k), as the per-user loop skips a metric that raises."""
+    for m in metrics:
+        for j, k_ in enumerate(ks):
+            if type(m) is NDCG:
+                cur, best = dcg[:, j], idcg[:, j]
+                good = best != 0                                    # ZeroDivisionError -> metric skipped for the user
+                vals = (cur[good] / best[good]).tolist()
+            else:
+                hits = hits_all[:, j]
+                if type(m) is Precision:
+                    good = n_rec[:, j] > 0
+                    vals = (hits[good] / n_rec[good, j]).tolist()
+                else:                                               # HitRatio, Recall: / number of positives
+                    den = n_pos_distinct if type(m) is HitRatio else n_pos
+                    good = den > 0
+                    vals = (hits[good] / den[good]).tolist()
+            acc = 0
+            for v in vals:                                          # same left-to-right float additions as the loop
+                acc += v
+            metric_sums[(m.name, k_)] = [acc, len(vals)]
+
+
+def _metric_results(metric_sums):
     return {m + f'@{k_}': round(metric_sums[(m, k_)][0] / metric_sums[(m, k_)][1], 4)
             if metric_sums[(m, k_)][1] > 0 else 0 for m, k_ in metric_sums}
+
+
+def _call_metrics(metric_sums, metrics, ks, recommendations, positives, best_item, relevancies):
+    """ranking_evaluation.py:223-246: every metric gets the arguments its __call__ names; an exception skips that
+    (metric, k) for the user."""
+    for m in metrics:
+        param_names = m.__call__.__code__.co_varnames
+        for k_ in ks:
+            params = dict()
+            for param_name in param_names:
+                if param_name == 'recommendations': params[param_name] = recommendations
+                elif param_name == 'relevant_recommendations': params[param_name] = positives
+                elif param_name == 'relevant_recommendation': params[param_name] = best_item
+                elif param_name == 'relevancies': params[param_name] = relevancies
+                elif param_name == 'k': params[param_name] = k_
+            try:
+                metric_sums[(m.name, k_)][0] += m(**params)
+                metric_sums[(m.name, k_)][1] += 1
+            except Exception:
+                pass
 
 
 # ------------------------------------------------------------------------------------------ the protocol
@@ -355,21 +394,256 @@ def ranking_evaluation(model, ds_test=None, n_test_users=None, k=10, n_pos_inter
         best_item = None if len(positives) == 0 else min(positives, key=lambda it: relevancies[it])
         if record is not None:
             record.append((users[u].item() if hasattr(users[u], 'item') else users[u], all_items, list(recommendations)))
-        for m in metrics:
-            param_names = m.__call__.__code__.co_varnames
-            for k_ in k:
-                params = dict()
-                for param_name in param_names:
-                    if param_name == 'recommendations': params[param_name] = recommendations
-                    elif param_name == 'relevant_recommendations': params[param_name] = positives
-                    elif param_name == 'relevant_recommendation': params[param_name] = best_item
-                    elif param_name == 'relevancies': params[param_name] = relevancies
-                    elif param_name == 'k': params[param_name] = k_
-                try:
-                    metric_sums[(m.name, k_)][0] += m(**params)
-                    metric_sums[(m.name, k_)][1] += 1
-                except Exception:
-                    pass
+        _call_metrics(metric_sums, metrics, k, recommendations, positives, best_item, relevancies)
 
-    return {m + f'@{k_}': round(metric_sums[(m, k_)][0] / metric_sums[(m, k_)][1], 4)
-            if metric_sums[(m, k_)][1] > 0 else 0 for m, k_ in metric_sums}
+    return _metric_results(metric_sums)
+
+
+# ------------------------------------------------------------------------------------------ recommendation_evaluation
+_TOPK_MAX = 2048            # longest list the models' full-catalog top-k (topk_batch) produces
+
+
+def _float32_from_order(o):
+    """Inverse of the order-preserving map float32 -> uint32 (the f2ord of the top-k kernels)."""
+    u = (o & 0x7fffffff) if o & 0x80000000 else (~o & 0xffffffff)
+    return np.array([u], np.uint32).view(np.float32)
+
+
+def _score_cut(model, threshold):
+    """recommend(..., interaction_threshold=t) keeps an item when its reported score is >= t.  The reported score is a
+    non-decreasing function of the float32 top-k score (CDAE: the score itself, so NumPy compares in float32; DMF: the
+    rescaled p, in float64 when the interaction bounds are NumPy scalars), so the kept items are those whose top-k score
+    is >= the smallest finite float32 whose reported score passes.  Found by bisection over the float32 values in
+    order, with the same NumPy comparison recommend() makes.  NaN when no finite float32 passes (no score is >= NaN)."""
+    def keeps(o):
+        with np.errstate(all='ignore'):
+            return bool(model._reported_scores(_float32_from_order(o))[0] >= threshold)
+    lo, hi = 0x00800000, 0xff7fffff             # order keys of -FLT_MAX and FLT_MAX
+    if not keeps(hi):
+        return float('nan')
+    while lo < hi:
+        mid = (lo + hi) // 2
+        if keeps(mid): hi = mid
+        else: lo = mid + 1
+    return float(_float32_from_order(lo)[0])
+
+
+def _fast_recommendation_evaluation(model, data, users, t_indptr, t_order, thr, n_pos, train_evaluation, seed, novelty,
+                                    low_threshold, metrics, ks, chunk, timings):
+    """The protocol of the per-user loop in recommendation_evaluation for the built-in metrics, with the top-k lists
+    and the per-user metric sums on the device.  Returns None when a corner case needs the general path (a negative
+    relevancy: the reference's ideal list then ranks the recommended items outside the evaluated set, which count 0,
+    above it)."""
+    import torch
+    t0 = time.perf_counter()
+    cand_off, cand, pos_off, pos, skipped, t_item, t_val = generate_candidates(
+        model, data, users, t_indptr, t_order, thr, n_pos, None, False, train_evaluation, seed)
+    metric_sums = {(m.name, k_): [0, 0] for m in metrics for k_ in ks}
+    active = np.flatnonzero(skipped == 0)
+    if len(active):
+        active = active[model._data.users_to_uids(users[active]) >= 0]     # recommend() asserts -> user skipped
+    n = len(active)
+    if n == 0:
+        return _metric_results(metric_sums)
+    t_item, t_val = t_item[:t_indptr[-1]], t_val[:t_indptr[-1]]
+
+    # every (user, item) pair as one integer key: the user's evaluation index and the item's code among the test items
+    codes, uniq = pd.factorize(t_item)
+    nc = max(len(uniq), 1)
+    code_index = pd.Index(uniq)
+    tkey = np.repeat(np.arange(len(users), dtype=np.int64), np.diff(t_indptr)) * nc + codes
+    srt = np.argsort(tkey, kind='stable')               # rows of one key stay in row order: the first comes first
+    tk = tkey[srt]
+    first = np.concatenate(([True], tk[1:] != tk[:-1]))
+    tkey_first, tval_first = tk[first], t_val[srt][first]
+
+    def members(off, flat):
+        """The active users' lists back to back: (items, evaluation index of their user, list lengths)."""
+        lens = (off[active + 1] - off[active]).astype(np.int64)
+        start = np.zeros(n, np.int64)
+        np.cumsum(lens[:-1], out=start[1:])
+        idx = np.arange(int(lens.sum()), dtype=np.int64) - np.repeat(start - off[active], lens)
+        return flat[idx], np.repeat(active.astype(np.int64), lens), lens
+    c_items, c_user, _ = members(cand_off, cand)
+    p_items, p_user, p_lens = members(pos_off, pos)
+    ekey = np.unique(c_user * nc + code_index.get_indexer(c_items))     # distinct items of every evaluated set C
+    pkey = np.unique(p_user * nc + code_index.get_indexer(p_items))     # distinct sampled positives
+    e_val = tval_first[np.searchsorted(tkey_first, ekey)]               # value of the user's first test row
+    if not (e_val >= 0).all():
+        return None
+    j = np.minimum(np.searchsorted(pkey, ekey), max(len(pkey) - 1, 0))
+    e_pos = (pkey[j] == ekey) if len(pkey) else np.zeros(len(ekey), bool)
+    e_row = np.searchsorted(active, ekey // nc)                         # row of the user among the active users
+    p_distinct = np.bincount(np.searchsorted(active, pkey // nc), minlength=n).astype(np.int64)
+    # gains 2 ** rel - 1 as the metric classes compute them (C library pow), once per distinct value
+    vals, inv = np.unique(e_val, return_inverse=True)
+    e_gain = np.array([2 ** float(v) - 1 for v in vals.tolist()], np.float64)[inv.ravel()]
+    ideal_off = np.zeros(n + 1, np.int64)
+    np.cumsum(np.bincount(e_row, minlength=n), out=ideal_off[1:])      # ekey is sorted by user: rows are contiguous
+    e_iid = np.asarray(model._data.items_to_iids(uniq[ekey % nc]), np.int64)
+    known = np.flatnonzero(e_iid >= 0)                                  # items the model can recommend
+    lut = known[np.argsort(e_row[known] * (int(model.n_items) + 1) + e_iid[known], kind='stable')]   # by (user, iid)
+    lut_off = np.zeros(n + 1, np.int64)
+    np.cumsum(np.bincount(e_row[lut], minlength=n), out=lut_off[1:])
+    K = max(ks)
+    disc = np.array([math.log2(2 + i) for i in range(K)], np.float64)
+    use_thr = low_threshold is not None
+    cut = _score_cut(model, low_threshold) if use_thr else 0.0
+    uids = np.asarray(model._data.users_to_uids(users[active]), np.int32)
+    t1 = time.perf_counter()
+
+    dev = model._dev
+
+    def up(a, dtype):
+        a = np.ascontiguousarray(a, dtype)
+        return torch.from_numpy(a if len(a) else np.zeros(1, dtype)).to(dev)   # never a NULL device pointer
+    d = {'uids': up(uids, np.int32), 'lut_off': up(lut_off, np.int64), 'lut_iid': up(e_iid[lut], np.int32),
+         'lut_gain': up(e_gain[lut], np.float64), 'lut_pos': up(e_pos[lut], np.uint8),
+         'ideal_off': up(ideal_off, np.int64), 'ideal_gain': up(e_gain, np.float64), 'disc': up(disc, np.float64),
+         'ks': up(ks, np.int32)}
+    nk = len(ks)
+    d_dcg = torch.empty((n, nk), dtype=torch.float64, device=dev)
+    d_idcg = torch.empty((n, nk), dtype=torch.float64, device=dev)
+    d_hits = torch.empty((n, nk), dtype=torch.int32, device=dev)
+    d_nrec = torch.empty((n, nk), dtype=torch.int32, device=dev)
+    lib, P = _lib.load(), _lib.t_ptr
+    ev = [] if timings is not None else None
+    with model._lock:
+        stream = model._stream                          # the stream libdrb enqueues on
+        for o in range(0, n, chunk):
+            c = min(chunk, n - o)
+            if ev is not None:
+                ev.append([torch.cuda.Event(enable_timing=True) for _ in range(3)])
+                ev[-1][0].record(stream)
+            o_i, o_s, o_n = model._topk_device_scores(d['uids'][o:o + c], K, novelty)
+            if ev is not None:
+                ev[-1][1].record(stream)
+            _lib.check(lib.drb_eval_topk_metrics(
+                model._ctx, c, P(o_i), P(o_s), K, P(o_n), int(use_thr), cut, P(d['lut_off'][o:]), P(d['lut_iid']),
+                P(d['lut_gain']), P(d['lut_pos']), P(d['ideal_off'][o:]), P(d['ideal_gain']), P(d['disc']), P(d['ks']),
+                nk, K, P(d_dcg[o:]), P(d_idcg[o:]), P(d_hits[o:]), P(d_nrec[o:])))
+            if ev is not None:
+                ev[-1][2].record(stream)
+        t2 = time.perf_counter()
+        dcg, idcg = d_dcg.cpu().numpy(), d_idcg.cpu().numpy()
+        hits, n_rec = d_hits.cpu().numpy(), d_nrec.cpu().numpy()
+    t3 = time.perf_counter()
+    _metric_sums_from_user_values(metric_sums, metrics, ks, dcg, idcg, hits, n_rec, p_lens, p_distinct)
+    res = _metric_results(metric_sums)
+    if timings is not None:
+        timings.update(host_protocol_s=(t1 - t0) + (time.perf_counter() - t3), launch_and_upload_s=t2 - t1,
+                       copy_back_s=t3 - t2, topk_ms=sum(a.elapsed_time(b) for a, b, _ in ev),
+                       metrics_kernel_ms=sum(b.elapsed_time(c_) for _, b, c_ in ev), n_users=n,
+                       per_user={'dcg': dcg, 'idcg': idcg, 'hits': hits, 'n_rec': n_rec, 'users': users[active]})
+    return res
+
+
+def recommendation_evaluation(model, ds_test=None, n_test_users=None, k=10, n_pos_interactions=None, novelty=False,
+                              ignore_low_predictions_threshold=None, metrics=None, max_concurrent_threads=4, seed=0,
+                              verbose=True, **kwds):
+    """Full-catalog recommendation metrics of every test user (DRecPy's recommendation_evaluation protocol, same
+    signature).  Returns {'<metric>@<k>': value}.
+
+    Test users are taken in order of first appearance in ds_test (the first n_test_users of them).  For test user idx:
+      1. rng = random.Random(seed + idx);
+      2. positives: the user's test rows, in row order, with value >= interaction_threshold (the model's, or the
+         `interaction_threshold` keyword); all of them if n_pos_interactions is None, else rng.sample(positives,
+         n_pos_interactions), and a user with fewer positives than that is skipped;
+      3. the evaluated set C: the sampled positives plus every test row of the user below the threshold (what
+         ranking_evaluation evaluates with n_neg_interactions=None, generate_negative_pairs=False); relevancy(item) =
+         the value of the user's first test row with that item if the item is in C, else 0;
+      4. a user the model was not trained on is skipped (model.recommend raises AssertionError);
+      5. recommendations = [item for _, item in model.recommend(user, n=max(k), novelty=novelty,
+         interaction_threshold=ignore_low_predictions_threshold)];
+      6. every metric gets the arguments its __call__ names: recommendations, relevant_recommendations (the sampled
+         positives), relevant_recommendation (the positive of lowest relevancy), relevancies (the relevancy of every
+         item of C and of the recommendations) and k; a metric that raises (no positives, an empty list, an ideal DCG
+         of 0) skips that (metric, k) for the user;
+      7. each result is round(sum / count, 4), or 0 when no user counted.
+    Default metrics: Precision, Recall, HitRatio and NDCG.  ds_test None (or the model's own dataset) evaluates on the
+    training set.  max_concurrent_threads and verbose are accepted for compatibility and not used.
+
+    Models with a full-catalog top-k on the device (CDAE, DMF) with integer raw item ids, the built-in metrics (strong
+    relevancy) and max(k) <= 2048 are evaluated `chunk` users at a time (keyword, default 8192): topk_batch, then
+    drb_eval_topk_metrics on the device computes each user's DCG, ideal DCG and hit counts; only those come back to the
+    host.  The result is the same dict as the per-user loop.  Anything else runs the per-user loop over
+    model.recommend, as do record= (a list that receives (user, C, recommendations) per evaluated user) and
+    force_python=True.  timings= (a dict) receives, from the device path, the wall time of its host, upload and copy
+    parts, the CUDA-event time of the top-k and of the metric kernel, and the per-user arrays with the evaluated users.
+    """
+    assert n_test_users is None or n_test_users > 0, f'The number of test users ({n_test_users}) should be > 0.'
+    assert n_pos_interactions is None or n_pos_interactions > 0, \
+        f'The number of positive interactions ({n_pos_interactions}) should be None or an integer > 0.'
+    interaction_threshold = kwds.get('interaction_threshold', model.interaction_threshold)
+    if type(k) is not list: k = [k]
+    for k_ in k: assert k_ > 0, f'k ({k_}) should be > 0.'
+
+    train_evaluation = False
+    if ds_test is None or ds_test is model.interaction_dataset or ds_test is getattr(model, '_data', None):
+        train_evaluation = True
+        ds_test = model.interaction_dataset
+    if metrics is None:
+        metrics = [Precision(), Recall(), HitRatio(), NDCG()]
+    assert isinstance(metrics, list), f'Expected "metrics" argument to be a list and found {type(metrics)}. ' \
+        f'Should contain instances of RankingMetricABC.'
+    for m in metrics:
+        assert hasattr(m, 'name') and callable(m), f'Expected metric {m} to be an instance of type RankingMetricABC.'
+
+    data = InteractionData.from_dataset(ds_test)
+    users, t_indptr, t_order = _group_by_user(data)
+    n_eval = len(users) if n_test_users is None else min(n_test_users, len(users))
+    users, t_indptr = users[:n_eval], np.ascontiguousarray(t_indptr[:n_eval + 1])
+    record = kwds.get('record', None)
+    n_top = max(k)
+
+    native_ids = np.issubdtype(data.item.dtype, np.integer)
+    fast = (native_ids and hasattr(model, 'topk_batch') and hasattr(model, '_topk_device_scores') and record is None
+            and not kwds.get('force_python', False) and n_top <= _TOPK_MAX
+            and all(type(m) in (HitRatio, NDCG, Precision, Recall) and getattr(m, 'strong_relevancy', True)
+                    for m in metrics))
+    if fast:
+        res = _fast_recommendation_evaluation(model, data, users, t_indptr, t_order, interaction_threshold,
+                                              n_pos_interactions, train_evaluation, seed, novelty,
+                                              ignore_low_predictions_threshold, metrics, k, int(kwds.get('chunk', 8192)),
+                                              kwds.get('timings'))
+        if res is not None:
+            return res
+
+    # ---- the per-user protocol (steps 1-3 through the same candidate generation as ranking_evaluation)
+    evaluated = []           # (index, C, sampled positives, test items, test values)
+    if native_ids:
+        cand_off, cand, pos_off, pos, skipped, t_item, t_val = generate_candidates(
+            model, data, users, t_indptr, t_order, interaction_threshold, n_pos_interactions, None, False,
+            train_evaluation, seed)
+        for u in np.flatnonzero(skipped == 0).tolist():
+            evaluated.append((u, cand[cand_off[u]:cand_off[u + 1]].tolist(), pos[pos_off[u]:pos_off[u + 1]].tolist(),
+                              t_item[t_indptr[u]:t_indptr[u + 1]].tolist(), t_val[t_indptr[u]:t_indptr[u + 1]].tolist()))
+    else:
+        for idx in range(n_eval):
+            sl = t_order[t_indptr[idx]:t_indptr[idx + 1]]
+            r_items, r_vals = data.item[sl].tolist(), data.interaction[sl].tolist()
+            tpos = [it for it, v in zip(r_items, r_vals) if v >= interaction_threshold]
+            res = _candidates_python(random.Random(seed + idx), list(zip(r_items, r_vals)), [], tpos, model.n_items,
+                                     interaction_threshold, n_pos_interactions, None, False, train_evaluation)
+            if res is not None:
+                evaluated.append((idx, res[0], res[1], r_items, r_vals))
+
+    metric_sums = {(m.name, k_): [0, 0] for m in metrics for k_ in k}
+    for u, all_items, positives, r_items, r_vals in evaluated:
+        user = users[u].item() if hasattr(users[u], 'item') else users[u]
+        try:
+            recs = model.recommend(user, n=n_top, novelty=novelty,
+                                   interaction_threshold=ignore_low_predictions_threshold)
+        except AssertionError:
+            continue                                        # user unknown to the model
+        recommendations = [item for _, item in recs]
+        first_val = {}
+        for it, v in zip(r_items, r_vals):
+            first_val.setdefault(it, v)
+        relevancies = {item: 0 for item in recommendations}
+        relevancies.update({item: (first_val.get(item) or 0) for item in all_items})
+        best_item = None if len(positives) == 0 else min(positives, key=lambda it: relevancies[it])
+        if record is not None:
+            record.append((user, list(all_items), recommendations))
+        _call_metrics(metric_sums, metrics, k, recommendations, positives, best_item, relevancies)
+    return _metric_results(metric_sums)

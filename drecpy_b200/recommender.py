@@ -280,6 +280,16 @@ class DeepRecommenderABC(ABC):
             scores = np.full((U, n), np.nan, np.float32)
         return items, scores, counts
 
+    def _topk_device_scores(self, uids, k, novelty):
+        """topk_batch(uids, k, novelty) as device tensors, with the scores in the form the top-k kernel produced them;
+        recommend() reports _reported_scores of them (used by recommendation_evaluation to apply its threshold on the
+        device exactly as recommend() applies it)."""
+        return self.topk_batch(uids, k, novelty, return_device=True)
+
+    def _reported_scores(self, scores):
+        """The scores recommend() reports, from a float32 numpy array of _topk_device_scores' scores."""
+        return scores
+
     def rank(self, user_id, item_ids, novelty=True, skip_invalid_items=True, **kwds):
         assert self.fitted is True, 'The model requires to be fitted before being able to make predictions.'
         assert self._data.user_to_uid(user_id) is not None, f'User {user_id} was not found.'

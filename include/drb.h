@@ -437,6 +437,24 @@ int drb_eval_metrics(int64_t n_groups, const int64_t* tab_beg, const int64_t* ta
                      const int64_t* p_end, const int64_t* p_key, const int64_t* ks, int32_t n_ks, int32_t n_threads,
                      double* dcg, double* idcg, int64_t* hits);
 
+/* The same per-user sums for full-catalog top-k lists that are still on the device (replaces the per-user metric calls
+ * of DRecPy/Evaluation/Processes/recommendation_evaluation.py:164-192 on model.recommend's list), enqueued on the
+ * context's stream without synchronising.  All pointers are device pointers.  User u's list is top_iid / top_score
+ * [u * ld .. + n_out[u]) as drb_cdae_topk / drb_dmf_topk leave it (internal item ids, descending scores); its valid
+ * prefix is the first min(n_out[u], k_max) entries, cut at the first score < (float)threshold when use_threshold != 0.
+ * lut_iid[lut_off[u] .. lut_off[u+1]) are the internal ids, sorted ascending, of the user's evaluated items with their
+ * gain lut_gain (2^rel - 1) and lut_pos != 0 for a sampled positive; ideal_gain[ideal_off[u] .. ideal_off[u+1]) are the
+ * gains of all the user's evaluated items (also those the model does not know); disc[i] = log2(2 + i) for i < k_max;
+ * ks[n_ks] the cut-offs, 1 <= ks[j] <= k_max <= ld.  Outputs [n][n_ks]: dcg / hits over the first min(ks[j], n_valid)
+ * entries, idcg over the largest min(ks[j], #ideal gains) gains in descending order, n_rec = min(ks[j], n_valid).  Bit
+ * for bit what drb_eval_metrics computes for the same valid prefix, with the evaluated items as test table and
+ * candidate list. */
+int drb_eval_topk_metrics(drb_ctx* ctx, int32_t n, const int32_t* top_iid, const float* top_score, int32_t ld,
+                          const int32_t* n_out, int32_t use_threshold, double threshold, const int64_t* lut_off,
+                          const int32_t* lut_iid, const double* lut_gain, const uint8_t* lut_pos,
+                          const int64_t* ideal_off, const double* ideal_gain, const double* disc, const int32_t* ks,
+                          int32_t n_ks, int32_t k_max, double* dcg, double* idcg, int32_t* hits, int32_t* n_rec);
+
 /* Leave-k-out split for every user at once (replaces DRecPy/Evaluation/Splits/leave_k_out.py:58-135: one
  * interaction_dataset.select('user == ...') plus rng.sample per user on a thread pool).  Rows are given grouped by
  * user in order of first appearance, each group in DataFrame order: group idx spans user_indptr[idx]..[idx+1].  User
