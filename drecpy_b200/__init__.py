@@ -8,7 +8,8 @@ from .sampler import PointSampler
 from .recommender import DeepRecommenderABC
 from .cdae import CDAE
 from .dmf import DMF
-from .evaluation import ranking_evaluation, recommendation_evaluation, HitRatio, NDCG, DCG, Precision, Recall
+from .evaluation import (ranking_evaluation, recommendation_evaluation, predictive_evaluation, HitRatio, NDCG, DCG,
+                         Precision, Recall, RMSE, MSE, MAE)
 from .splits import leave_k_out
 from .early_stopping import MaxValidationValueRule
 from .loss_tracker import LossTracker
@@ -16,5 +17,6 @@ from .loss_tracker import LossTracker
 InteractionDataset = InteractionData
 
 __all__ = ['InteractionData', 'InteractionDataset', 'synthetic_interactions', 'synthetic_item_shard', 'PointSampler', 'DeepRecommenderABC', 'leave_k_out',
-           'CDAE', 'DMF', 'ranking_evaluation', 'recommendation_evaluation', 'HitRatio', 'NDCG', 'DCG', 'Precision', 'Recall',
+           'CDAE', 'DMF', 'ranking_evaluation', 'recommendation_evaluation', 'predictive_evaluation', 'HitRatio', 'NDCG', 'DCG',
+           'Precision', 'Recall', 'RMSE', 'MSE', 'MAE',
            'MaxValidationValueRule', 'LossTracker']

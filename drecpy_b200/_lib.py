@@ -120,6 +120,7 @@ SIGNATURES = {
     'drb_cdae_topk': (C.c_int, [vp, vp, i32, i32, i32, vp, vp, vp]),
     'drb_cdae_topk_exact': (C.c_int, [vp, vp, i32, i32, i32, vp, vp, vp]),
     'drb_cdae_predict_all': (C.c_int, [vp, vp, i32, vp]),
+    'drb_cdae_predict_pairs': (C.c_int, [vp, vp, i32, vp, vp, vp, i32, vp]),
     'drb_dmf_layout': (C.c_int, [i32, i32, vp, i32, vp, i32, P(DmfLayout)]),
     'drb_dmf_workspace_bytes': (i64, [i32, i32, vp, i32, vp, i32, i32]),
     'drb_dmf_create': (C.c_int, [vp, P(DmfDesc), P(vp)]),
@@ -129,6 +130,7 @@ SIGNATURES = {
     'drb_dmf_grads_buffer': (C.c_int, [vp, P(vp), P(i64)]),
     'drb_dmf_step_host': (C.c_int, [vp, vp, vp, vp, i32, P(DmfStepArgs), vp]),
     'drb_dmf_forward_pairs': (C.c_int, [vp, vp, vp, i32, vp]),
+    'drb_dmf_predict_pairs': (C.c_int, [vp, vp, i32, vp, vp, vp, i32, vp]),
     'drb_dmf_rank_candidates': (C.c_int, [vp, vp, i32, vp, vp, i32, i32, vp, vp, vp]),
     'drb_dmf_invalidate_cache': (C.c_int, [vp]),
     'drb_dmf_topk_scratch_bytes': (i64, [vp, i32]),

@@ -545,6 +545,17 @@ class CDAE(DeepRecommenderABC):
             predictions = out[:self.n_items].cpu().numpy()
         return predictions if iid is None else predictions[iid]
 
+    def predict_batch(self, user_ids, item_ids, skip_errors=False, chunk=1 << 22):
+        if getattr(self, '_sharded', False) or getattr(self, '_shard_csr', None) is not None:
+            raise NotImplementedError('predict_batch: an item-sharded CDAE holds only its shard of the output layer, '
+                                      'so its scores are not predict() values')
+        return super().predict_batch(user_ids, item_ids, skip_errors, chunk)
+
+    def _launch_predict_pairs(self, users, pair_off, pair_iid, pair_dst, out):
+        _lib.check(_lib.load().drb_cdae_predict_pairs(self._native, _lib.t_ptr(users), users.numel(),
+                                                      _lib.t_ptr(pair_off), _lib.t_ptr(pair_iid), _lib.t_ptr(pair_dst),
+                                                      out.numel(), _lib.t_ptr(out)))
+
     def hidden(self, uids):
         torch = self._torch
         with self._lock:

@@ -33,6 +33,24 @@ struct Carver {  // bump allocator over the caller-provided workspace (256-byte 
 // upper bound on the row blocks k_dz1 / k_colpart use for any batch <= max_batch (8 rows per block, 4 below 2048 rows)
 int colpart_blocks(int max_batch) { return std::max((max_batch + 7) / 8, (std::min(max_batch, 2047) + 3) / 4); }
 
+// Argument checks of a pair-scoring call (drb_cdae_predict_pairs / drb_dmf_predict_pairs): host-side ones, then the
+// device arrays are checked by one kernel whose verdict (one int in `flag_dev`, a scratch word) is read back here.
+int pair_args_check(drb_ctx* ctx, const char* fn, const PairArgs& p, int n_users, int n_items, int* flag_dev) {
+  if (p.n_u < 0 || p.n < 0) return drb_fail(DRB_E_INVALID, "%s: n_users %d, n %d", fn, p.n_u, p.n);
+  if (!p.users || !p.pair_off || (p.n > 0 && (!p.pair_iid || !p.pair_dst)))
+    return drb_fail(DRB_E_INVALID, "%s: NULL argument", fn);
+  int r = launch_pair_args_check(ctx, p, n_users, n_items, flag_dev);
+  if (r) return r;
+  int bad = 0;
+  DRB_CUDA_TRY(ctx, cudaMemcpyAsync(&bad, flag_dev, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  DRB_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (bad & 1) return drb_fail(DRB_E_INVALID, "%s: a user id is outside [0, %d)", fn, n_users);
+  if (bad & 2) return drb_fail(DRB_E_INVALID, "%s: pair_off must rise from 0 to n = %d", fn, p.n);
+  if (bad & 4) return drb_fail(DRB_E_INVALID, "%s: an item id is outside [0, %d)", fn, n_items);
+  if (bad & 8) return drb_fail(DRB_E_INVALID, "%s: an output position is outside [0, %d)", fn, p.n);
+  return DRB_OK;
+}
+
 int gemm_splits(const drb_ctx* ctx, int M, int N, int Kred) {
   const int tiles = ((M + 127) / 128) * ((N + 127) / 128);
   int s = (2 * ctx->sm_count + tiles - 1) / tiles;
@@ -939,6 +957,25 @@ int drb_cdae_predict_all(drb_cdae* m, const int32_t* uids, int32_t n, float* out
   return DRB_OK;
 }
 
+int drb_cdae_predict_pairs(drb_cdae* m, const int32_t* users, int32_t n_users, const int64_t* pair_off,
+                           const int32_t* pair_iid, const int32_t* pair_dst, int32_t n, float* out) {
+  if (!m || (n > 0 && !out)) return drb_fail(DRB_E_INVALID, "drb_cdae_predict_pairs: NULL argument");
+  const PairArgs p{users, n_users, pair_off, pair_iid, pair_dst, n};
+  if (n_users == 0 && n == 0) return DRB_OK;
+  int r = pair_args_check(m->ctx, "drb_cdae_predict_pairs", p, m->d.n_users, m->d.n_items,
+                          reinterpret_cast<int*>(m->ws.dz));
+  if (r) return r;
+  for (int32_t o = 0; o < n_users; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, n_users - o);
+    // h exactly as cdae_scores_chunk forms it for drb_cdae_predict_all
+    if ((r = cdae_hidden_into(m, users + o, c, nullptr, nullptr, 1.0f, m->ws.h))) return r;
+    if ((r = launch_cdae_pair_scores(m->ctx, p, o, c, m->ws.h, m->d.params + m->L.off_w2t, m->d.params + m->L.off_b2,
+                                     m->L.ld, out)))
+      return r;
+  }
+  return DRB_OK;
+}
+
 int drb_cdae_rank_candidates(drb_cdae* m, const int32_t* uids, int32_t n, const int32_t* cand,
                              const int32_t* cand_count, int32_t max_cand, int32_t novelty, int32_t* out_iid,
                              float* out_score, int32_t* n_out) {
@@ -1744,6 +1781,28 @@ int drb_dmf_topk(drb_dmf* m, const int32_t* uids, int32_t n, int32_t k, int32_t 
     t.out_iid = b_iid; t.out_score = b_score; t.n_out = n_out + o;
     if ((r = launch_dmf_topk_fallback(ctx, t, c, m->tw[0].act[lu], m->tw[0].ld[lu], m->item_rep, ldl, width, S.fb_rows,
                                       S.fb_users, S.fb_count, kDmfTopkFallbackRows)))
+      return r;
+  }
+  return DRB_OK;
+}
+
+int drb_dmf_predict_pairs(drb_dmf* m, const int32_t* users, int32_t n_users, const int64_t* pair_off,
+                          const int32_t* pair_iid, const int32_t* pair_dst, int32_t n, float* p_out) {
+  if (!m || (n > 0 && !p_out)) return drb_fail(DRB_E_INVALID, "drb_dmf_predict_pairs: NULL argument");
+  const PairArgs p{users, n_users, pair_off, pair_iid, pair_dst, n};
+  if (n_users == 0 && n == 0) return DRB_OK;
+  int r = pair_args_check(m->ctx, "drb_dmf_predict_pairs", p, m->d.n_users, m->d.n_items,
+                          reinterpret_cast<int*>(m->rank_scratch));
+  if (r) return r;
+  const int lu = m->tw[0].n_layers - 1, li = m->tw[1].n_layers - 1;
+  if ((r = dmf_refresh_item_rep(m))) return r;
+  for (int32_t o = 0; o < n_users; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, n_users - o);
+    // a tower row depends on its own id only (one CTA per row in the gather, splits = 1 in the layer GEMMs), so the
+    // rows equal those drb_dmf_forward_pairs computes for the same user / item
+    if ((r = dmf_tower_fwd(m, 0, users + o, c))) return r;
+    if ((r = launch_dmf_pair_head(m->ctx, p, o, c, m->tw[0].act[lu], m->tw[0].ld[lu], m->item_rep, m->tw[1].ld[li],
+                                  m->tw[0].width[lu], p_out)))
       return r;
   }
   return DRB_OK;

@@ -295,4 +295,21 @@ int launch_dmf_topk_filter(drb_ctx* ctx, const DmfFilterArgs& a);
 int launch_dmf_topk_fallback(drb_ctx* ctx, const TopkArgs& a, int n, const float* urep, int ld_u, const float* irep,
                              int ld_i, int width, float* rows, int32_t* fb_users, int32_t* fb_count, int fb_max);
 
+// ------------------------------------------------------------------ predict.cu (K11: (user, item) pair scores)
+// pairs grouped by user: user b owns pairs [pair_off[b], pair_off[b + 1]); pair q scores item pair_iid[q] into
+// out[pair_dst[q]]
+struct PairArgs {
+  const int32_t* users; int n_u;
+  const int64_t* pair_off; const int32_t* pair_iid; const int32_t* pair_dst; int n;
+};
+// *bad_dev = OR of: 1 user id outside [0, n_users), 2 pair_off not 0 .. n non-decreasing, 4 item id outside
+// [0, n_items), 8 output position outside [0, n)
+int launch_pair_args_check(drb_ctx* ctx, const PairArgs& p, int n_users, int n_items, int* bad_dev);
+// users [u0, u0 + c) of the CSR, h [c][ld] their hidden rows (row j = user u0 + j)
+int launch_cdae_pair_scores(drb_ctx* ctx, const PairArgs& p, int u0, int c, const float* h, const float* w2t,
+                            const float* b2, int ld, float* out);
+// users [u0, u0 + c), urep [c][ld_u] their user-tower rows, irep [n_items][ld_i] the item-tower cache
+int launch_dmf_pair_head(drb_ctx* ctx, const PairArgs& p, int u0, int c, const float* urep, int ld_u,
+                         const float* irep, int ld_i, int width, float* out);
+
 #endif

@@ -287,6 +287,12 @@ class DMF(DeepRecommenderABC):
         if uid is None or iid is None: return None
         return self._rescale_value(self.forward_pairs([uid], [iid])[0])
 
+    def _launch_predict_pairs(self, users, pair_off, pair_iid, pair_dst, out):
+        self._sync_item_cache()                       # the item side comes from the catalog cache
+        _lib.check(_lib.load().drb_dmf_predict_pairs(self._native, _lib.t_ptr(users), users.numel(),
+                                                     _lib.t_ptr(pair_off), _lib.t_ptr(pair_iid), _lib.t_ptr(pair_dst),
+                                                     out.numel(), _lib.t_ptr(out)))
+
     def _sync_item_cache(self):
         # the library caches the item tower of the whole catalog between steps; in-place writes to the arena from
         # Python (weight injection, _revert_weights) bump the tensor version -> tell it

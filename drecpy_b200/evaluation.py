@@ -10,6 +10,10 @@ Models without rank_batch (any object with .rank) and non-integer raw ids go thr
 recommendation_evaluation (DRecPy/Evaluation/Processes/recommendation_evaluation.py:18-192, restated: see its
 docstring) evaluates the full-catalog top-k of every test user; for CDAE / DMF the lists stay on the device and
 drb_eval_topk_metrics reduces them to per-user DCG / ideal DCG / hit counts there.
+
+predictive_evaluation (DRecPy/Evaluation/Processes/predictive_evaluation.py:7-65 with Metrics/regression.py, restated:
+see its docstring) computes RMSE / MSE / MAE of model.predict over the test rows; CDAE and DMF score all rows in one
+predict_batch call (drb_cdae_predict_pairs / drb_dmf_predict_pairs).
 """
 import math
 import os
@@ -647,3 +651,133 @@ def recommendation_evaluation(model, ds_test=None, n_test_users=None, k=10, n_po
             record.append((user, list(all_items), recommendations))
         _call_metrics(metric_sums, metrics, k, recommendations, positives, best_item, relevancies)
     return _metric_results(metric_sums)
+
+
+# ------------------------------------------------------------------------------------------ predictive_evaluation
+class PredictiveMetricABC:
+    @property
+    def name(self):
+        return self.__class__.__name__
+
+
+class MSE(PredictiveMetricABC):
+    """Mean squared error, in float64 (sklearn.metrics.mean_squared_error for one output)."""
+
+    def __call__(self, y_true, y_pred):
+        d = np.asarray(y_true, np.float64) - np.asarray(y_pred, np.float64)
+        return float(np.mean(d ** 2))
+
+
+class RMSE(PredictiveMetricABC):
+    """Square root of MSE."""
+
+    def __call__(self, y_true, y_pred):
+        return float(np.sqrt(MSE()(y_true, y_pred)))
+
+
+class MAE(PredictiveMetricABC):
+    """Mean absolute error, in float64 (sklearn.metrics.mean_absolute_error for one output)."""
+
+    def __call__(self, y_true, y_pred):
+        return float(np.mean(np.abs(np.asarray(y_true, np.float64) - np.asarray(y_pred, np.float64))))
+
+
+_PAIR_KERNELS = ('k_cdae_pair_scores', 'k_dmf_pair_head')
+
+
+def _fast_predictive_evaluation(model, data, count_none_predictions, n_test_predictions, skip_errors, chunk, timings):
+    """The rows, predictions and selection of the per-row loop in predictive_evaluation, with one predict_batch call
+    over the rows that loop would predict.  Returns (y_true, y_pred) as float64 arrays."""
+    t0 = time.perf_counter()
+    uids, iids = model._pair_ids(data.user, data.item)
+    none = (uids < 0) | (iids < 0)                         # predict() returns None (skip_errors) or raises
+    if not skip_errors and none.any():
+        first = int(np.argmax(none))
+        if n_test_predictions is None or first < n_test_predictions:     # the loop gets there before its cap
+            model.predict(data.user[first], data.item[first], skip_errors=False)   # raises predict()'s AssertionError
+    rows = np.arange(len(data)) if count_none_predictions else np.flatnonzero(~none)
+    if n_test_predictions is not None:
+        rows = rows[:n_test_predictions]
+    known = rows[~none[rows]]
+    t1 = time.perf_counter()
+    prof = timings is not None and getattr(model, '_ctx', None) is not None
+    if prof:
+        _lib.profile_read(model._ctx)                       # drop older records
+        _lib.check(_lib.load().drb_ctx_profile_enable(model._ctx, 1))
+    try:
+        pred = model.predict_batch(data.user[known], data.item[known], skip_errors=True, chunk=chunk)
+    finally:
+        if prof:
+            kernels = _lib.profile_read(model._ctx)
+            _lib.check(_lib.load().drb_ctx_profile_enable(model._ctx, 0))
+    t2 = time.perf_counter()
+    y_pred = np.zeros(len(rows), np.float64)
+    y_pred[~none[rows]] = pred
+    y_true = np.asarray(data.interaction[rows], np.float64)
+    if timings is not None:
+        timings.update(host_select_s=t1 - t0, predict_batch_s=t2 - t1, n_rows=len(rows), n_predicted=len(known))
+        if prof:
+            timings.update(kernels_ms=kernels,
+                           pair_kernel_ms=sum(v[0] for k, v in kernels.items() if k in _PAIR_KERNELS),
+                           user_side_kernel_ms=sum(v[0] for k, v in kernels.items() if k not in _PAIR_KERNELS))
+    return y_true, y_pred
+
+
+def predictive_evaluation(model, ds_test=None, count_none_predictions=False, n_test_predictions=None, skip_errors=True,
+                          metrics=None, verbose=True, **kwds):
+    """Regression metrics of model.predict over the rows of ds_test (DRecPy's predictive_evaluation protocol, same
+    signature).  Returns {metric.name: value}.
+
+    The protocol:
+      1. ds_test None evaluates on the model's training data (model.interaction_dataset);
+      2. the rows of ds_test are taken in row order; row (user, item, value) gets
+         prediction = model.predict(user, item, skip_errors=skip_errors), so with skip_errors=False an unknown user or
+         item raises predict()'s AssertionError;
+      3. a prediction of None (an unknown user or item, with skip_errors) is skipped, or counted as a prediction of 0
+         when count_none_predictions;
+      4. y_true collects the values and y_pred the predictions of the counted rows; after n_test_predictions counted
+         rows (when given) no further row is predicted;
+      5. every metric is computed on y_true / y_pred as float64 NumPy arrays: MSE = np.mean((y_true - y_pred) ** 2),
+         RMSE = its np.sqrt, MAE = np.mean(np.abs(y_true - y_pred)) (sklearn's operations for one output);
+      6. the result is {m.name: round(m(y_true, y_pred), 4)} in the order of metrics.
+    Default metrics: RMSE and MSE.  verbose is accepted for compatibility and not used.
+
+    Models with predict_batch (CDAE, DMF) make one predict_batch call over the rows step 4 counts (`chunk` pairs per
+    device call, keyword) and return the same dict as the per-row loop, from the same y_pred bit for bit.  force_python=
+    True runs the per-row loop.  timings= (a dict) receives y_true and y_pred from either path and, from the batched
+    path, the wall time of its host selection and of predict_batch, and the CUDA-event time of every kernel launched
+    (kernels_ms: {name: (ms, launches)}), summed into pair_kernel_ms (the pair kernels) and user_side_kernel_ms (the
+    hidden layer / towers and the argument check).
+    """
+    assert n_test_predictions is None or n_test_predictions > 0, \
+        f'The number of test predictions ({n_test_predictions}) should be > 0.'
+    if metrics is None:
+        metrics = [RMSE(), MSE()]
+    assert isinstance(metrics, list), f'Expected "metrics" argument to be a list and found {type(metrics)}. ' \
+        f'Should contain instances of PredictiveMetricABC.'
+    for m in metrics:
+        assert hasattr(m, 'name') and callable(m), f'Expected metric {m} to be an instance of type PredictiveMetricABC.'
+    if ds_test is None:
+        ds_test = model.interaction_dataset
+    data = InteractionData.from_dataset(ds_test)
+    timings = kwds.get('timings')
+
+    if hasattr(model, 'predict_batch') and hasattr(model, '_pair_ids') and not kwds.get('force_python', False):
+        y_true, y_pred = _fast_predictive_evaluation(model, data, count_none_predictions, n_test_predictions,
+                                                     skip_errors, int(kwds.get('chunk', 1 << 22)), timings)
+    else:
+        t_list, p_list = [], []
+        for user, item, value in zip(data.user.tolist(), data.item.tolist(), data.interaction.tolist()):
+            prediction = model.predict(user, item, skip_errors=skip_errors)
+            if prediction is None:
+                if not count_none_predictions:
+                    continue
+                prediction = 0
+            t_list.append(value)
+            p_list.append(prediction)
+            if n_test_predictions is not None and len(p_list) >= n_test_predictions:
+                break
+        y_true, y_pred = np.asarray(t_list, np.float64), np.asarray(p_list, np.float64)
+    if timings is not None:
+        timings.update(y_true=y_true, y_pred=y_pred)
+    return {m.name: round(m(y_true, y_pred), 4) for m in metrics}

@@ -223,12 +223,74 @@ class DeepRecommenderABC(ABC):
         prediction = None
         try:
             uid, iid = ds.user_to_uid(user_id), ds.item_to_iid(item_id)
-            prediction = self._predict(uid, iid, **kwds)
+            # _predict(uid, None) is the full score row (CDAE); an unknown item has no prediction
+            prediction = self._predict(uid, iid, **kwds) if uid is not None and iid is not None else None
             if prediction is None:
                 raise Exception(f'Failed to predict(user_id={user_id}, item_id={item_id}): None was returned.')
         except Exception as e:
             if not skip_errors: raise e
         return prediction
+
+    def predict_batch(self, user_ids, item_ids, skip_errors=False, chunk=1 << 22):
+        """Batched predict() over raw ids: element r is predict(user_ids[r], item_ids[r], skip_errors), bit for bit and
+        with the same dtype; where predict() returns None it is NaN.  With skip_errors=False the first pair with an
+        unknown user or item raises the AssertionError predict() raises for it.  Pairs go to the device `chunk` at a
+        time, grouped by user there (a stable sort by internal uid), so each distinct user's side of the model is
+        computed once per chunk and each pair is scored against one catalog row (drb_*_predict_pairs)."""
+        assert self.fitted is True, 'The model requires to be fitted before being able to make predictions.'
+        user_ids, item_ids = np.asarray(user_ids), np.asarray(item_ids)
+        assert user_ids.shape == item_ids.shape and user_ids.ndim == 1, \
+            f'predict_batch: user_ids and item_ids must be 1-d and of equal length ({user_ids.shape} != {item_ids.shape})'
+        n = len(user_ids)
+        uids, iids = self._pair_ids(user_ids, item_ids)
+        bad = (uids < 0) | (iids < 0)
+        if not skip_errors and bad.any():
+            r = int(np.argmax(bad))
+            if uids[r] < 0: raise AssertionError(f'User {user_ids[r]} was not found.')
+            raise AssertionError(f'Item {item_ids[r]} was not found.')
+        chunk = max(1, int(chunk))
+        if not bad.any() and n <= chunk:
+            raw = self._predict_pairs(uids, iids)
+        else:
+            raw = np.full(n, np.nan, np.float32)
+            ok = np.flatnonzero(~bad)
+            for o in range(0, len(ok), chunk):
+                sel = ok[o:o + chunk]
+                raw[sel] = self._predict_pairs(uids[sel], iids[sel])
+        return self._reported_scores(raw)
+
+    def _pair_ids(self, user_ids, item_ids):
+        """Internal (uid, iid) int32 arrays of raw id arrays; -1 where an id is unknown."""
+        if len(user_ids) == 0:
+            return np.zeros(0, np.int32), np.zeros(0, np.int32)
+        return (np.asarray(self._data.users_to_uids(user_ids)).astype(np.int32),
+                np.asarray(self._data.items_to_iids(item_ids)).astype(np.int32))
+
+    def _predict_pairs(self, uids, iids):
+        """float32 scores (as the model computes them before _reported_scores) of known (uid, iid) pairs, in order."""
+        torch = self._torch
+        n = len(uids)
+        if n == 0:
+            return np.zeros(0, np.float32)
+        with self._lock:
+            d_u = torch.from_numpy(np.ascontiguousarray(uids, np.int32)).to(self._dev)
+            d_i = torch.from_numpy(np.ascontiguousarray(iids, np.int32)).to(self._dev)
+            s_u, order = torch.sort(d_u, stable=True)
+            users, counts = torch.unique_consecutive(s_u, return_counts=True)
+            off = torch.zeros(users.numel() + 1, dtype=torch.int64, device=self._dev)
+            torch.cumsum(counts, 0, out=off[1:])
+            p_iid = d_i[order].contiguous()
+            p_dst = order.to(torch.int32)
+            out = torch.empty(n, dtype=torch.float32, device=self._dev)
+            self._launch_predict_pairs(users.to(torch.int32).contiguous(), off, p_iid, p_dst, out)
+            host = torch.empty(n, dtype=torch.float32, pin_memory=True)
+            host.copy_(out, non_blocking=True)
+            torch.cuda.current_stream(self._dev).synchronize()
+            return host.numpy()
+
+    def _launch_predict_pairs(self, users, pair_off, pair_iid, pair_dst, out):
+        """Enqueue drb_*_predict_pairs on device tensors (users int32, pair_off int64, pair_iid / pair_dst int32)."""
+        raise NotImplementedError(f'{self.__class__.__name__} has no batched pair scoring')
 
     def recommend(self, user_id, n=None, novelty=True, interaction_threshold=None, **kwds):
         assert self.fitted is True, 'The model requires to be fitted before being able to make predictions.'

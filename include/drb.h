@@ -277,6 +277,14 @@ int drb_cdae_topk_exact(drb_cdae* m, const int32_t* uids, int32_t n, int32_t k, 
                         int32_t* out_iid, float* out_score, int32_t* n_out);
 /* Dense scores for n users over all items: out[n x items_pad] (cdae.py:84-88 with iid=None). */
 int drb_cdae_predict_all(drb_cdae* m, const int32_t* uids, int32_t n, float* out);
+/* Scores of n (user, item) pairs.  replaces: recommender_abc.py:354-383 -> cdae.py:84-88 (_predict: the user's whole
+ * score row, then one element of it) once per pair.  Pairs are grouped by user: users[n_users] internal uids, user b
+ * owns pairs [pair_off[b], pair_off[b+1]) (pair_off[0] = 0, pair_off[n_users] = n, non-decreasing), pair q scores
+ * internal item pair_iid[q] into out[pair_dst[q]].  All device pointers; the call synchronises the context's stream
+ * once, to check the arguments (DRB_E_INVALID for an id or position out of range or a bad pair_off).  Every value is
+ * bit for bit the element drb_cdae_predict_all gives for that user and item. */
+int drb_cdae_predict_pairs(drb_cdae* m, const int32_t* users, int32_t n_users, const int64_t* pair_off,
+                           const int32_t* pair_iid, const int32_t* pair_dst, int32_t n, float* out);
 
 /* ------------------------------------------------------------------ DMF
  * Tower l has kernel [in_l, out_l] (row stride ld_l = out_l rounded up to a multiple of 4) and bias [ld_l].
@@ -342,6 +350,12 @@ int drb_dmf_step_host(drb_dmf* m, const int32_t* uids, const int32_t* iids, cons
 int drb_dmf_loss_buffer(drb_dmf* m, float** ptr);
 /* p[n] = max(1e-6, cos(user tower(uid), item tower(iid))) for n pairs (dmf.py:88-96, un-rescaled). device. */
 int drb_dmf_forward_pairs(drb_dmf* m, const int32_t* uids, const int32_t* iids, int32_t n, float* p_out);
+/* The same p for n pairs grouped by user, with the arguments of drb_cdae_predict_pairs.  replaces: recommender_abc.py:
+ * 354-383 -> dmf.py:101-106 (_predict: both towers for one pair) once per pair.  The user tower runs once per entry of
+ * users; the item side comes from the item-tower cache of drb_dmf_rank_candidates.  Every value is bit for bit what
+ * drb_dmf_forward_pairs gives for that pair (un-rescaled). */
+int drb_dmf_predict_pairs(drb_dmf* m, const int32_t* users, int32_t n_users, const int64_t* pair_off,
+                          const int32_t* pair_iid, const int32_t* pair_dst, int32_t n, float* p_out);
 /* replaces: recommender_abc.py:454-461 (one _predict per candidate + nlargest).  Same contract as
  * drb_cdae_rank_candidates; scores are the un-rescaled p (rescaling is monotone, done by the host). */
 int drb_dmf_rank_candidates(drb_dmf* m, const int32_t* uids, int32_t n, const int32_t* cand,
