@@ -34,6 +34,11 @@ class CdaeDesc(C.Structure):
                 ('output_mode', i32), ('neg_per_group', i32), ('neg_groups', i32)]
 
 
+class OptimDesc(C.Structure):
+    _fields_ = [('kind', i32), ('momentum', f32), ('nesterov', i32), ('rho', f32), ('centered', i32), ('beta1', f32),
+                ('beta2', f32), ('epsilon', f32), ('amsgrad', i32), ('decay', f32), ('third_state', vp)]
+
+
 class CdaeStepArgs(C.Structure):
     _fields_ = [('learning_rate', f32), ('beta1', f32), ('beta2', f32), ('epsilon', f32), ('reg_rate', f32),
                 ('t', i32 * 5), ('philox_seed', u64), ('philox_step', u64), ('global_batch', i32),
@@ -106,6 +111,7 @@ SIGNATURES = {
     'drb_cdae_workspace_bytes_sampled': (i64, [i32, i32, i32, i32]),
     'drb_cdae_create': (C.c_int, [vp, P(CdaeDesc), P(vp)]),
     'drb_cdae_destroy': (C.c_int, [vp]),
+    'drb_cdae_set_optimizer': (C.c_int, [vp, P(OptimDesc)]),
     'drb_cdae_step': (C.c_int, [vp, vp, vp, vp, i32, P(CdaeStepArgs), vp]),
     'drb_cdae_step_phases': (C.c_int, [vp, vp, vp, vp, i32, P(CdaeStepArgs), vp, i32]),
     'drb_cdae_label_count_buffer': (C.c_int, [vp, P(vp), P(i64)]),
@@ -125,6 +131,7 @@ SIGNATURES = {
     'drb_dmf_workspace_bytes': (i64, [i32, i32, vp, i32, vp, i32, i32]),
     'drb_dmf_create': (C.c_int, [vp, P(DmfDesc), P(vp)]),
     'drb_dmf_destroy': (C.c_int, [vp]),
+    'drb_dmf_set_optimizer': (C.c_int, [vp, P(OptimDesc)]),
     'drb_dmf_step': (C.c_int, [vp, vp, vp, vp, i32, P(DmfStepArgs), vp]),
     'drb_dmf_step_phases': (C.c_int, [vp, vp, vp, vp, i32, P(DmfStepArgs), vp, i32, i32]),
     'drb_dmf_grads_buffer': (C.c_int, [vp, P(vp), P(i64)]),

@@ -22,7 +22,7 @@ import random
 
 import numpy as np
 
-from . import _lib
+from . import _lib, optimizers
 from .parallel import DataParallel, data_parallel_step
 from .recommender import DeepRecommenderABC
 from .sampler import PointSampler
@@ -47,6 +47,8 @@ class UniformUserSampler:
 
 
 class CDAE(DeepRecommenderABC):
+    _SET_OPTIMIZER = 'drb_cdae_set_optimizer'
+
     def __init__(self, hidden_factors=50, corruption_level=0.2, loss='bce', **kwds):
         super(CDAE, self).__init__(**kwds)
         self.hidden_factors = hidden_factors
@@ -125,7 +127,7 @@ class CDAE(DeepRecommenderABC):
         self._torch = torch
         self.n_users, self.n_items, self.n_rows = int(n_users), int(n_items), int(shard_csr[1].shape[0])
         self.min_interaction, self.max_interaction = 0, 5
-        self.optimizer = {'learning_rate': learning_rate, 'beta_1': 0.9, 'beta_2': 0.999, 'epsilon': 1e-7}
+        self.optimizer = optimizers.parse(kwds.pop('optimizer', None), learning_rate)
         self._step = 0
         self.epoch_weights = {}
         idx = shard_csr[1]                                   # numpy, or a torch tensor already on this rank's GPU
@@ -143,8 +145,7 @@ class CDAE(DeepRecommenderABC):
         self._L = L
         dev = self._dev
         self._params = torch.zeros(L.total, dtype=torch.float32, device=dev)
-        self._adam_m = torch.zeros_like(self._params)
-        self._adam_v = torch.zeros_like(self._params)
+        self._alloc_optimizer_slots()
         self._grads = torch.zeros_like(self._params)
         K, I, U = self.hidden_factors, self.n_items, self.n_users
         gen = torch.Generator().manual_seed(abs(int(self.seed)) if self.seed is not None else random.getrandbits(62))
@@ -238,6 +239,7 @@ class CDAE(DeepRecommenderABC):
         _lib.check(lib.drb_cdae_dz1_buffer(self._native, C.byref(ptr), C.byref(cnt)))
         off = ptr.value - self._workspace.data_ptr()
         self._dz1 = self._workspace[off:off + 4 * cnt.value].view(torch.float32).view(-1, L.ld)
+        self._apply_optimizer()
 
     @staticmethod
     def _restrict_columns(csr, lo, hi):
@@ -300,7 +302,8 @@ class CDAE(DeepRecommenderABC):
     def step_args(self, reg_rate):
         o = self.optimizer
         a = _lib.CdaeStepArgs()
-        a.learning_rate, a.beta1, a.beta2, a.epsilon = o['learning_rate'], o['beta_1'], o['beta_2'], o['epsilon']
+        a.learning_rate = o['learning_rate']       # the rest of the optimizer is the model's drb_optim_desc
+        a.beta1, a.beta2, a.epsilon = o.get('beta_1', 0.9), o.get('beta_2', 0.999), o.get('epsilon', 1e-7)
         a.reg_rate = reg_rate
         s = self._step
         for j in range(5):

@@ -230,6 +230,8 @@ struct drb_cdae {
   bool reg_slots_clear;                   // the three reg_part slots were zeroed in PREP (split UPDATE of this step)
   int n2, batch_pad;   // tcgen05 path: N of the backward GEMMs (hidden + ones feature, rounded to 16), padded batch
   float* z_dbg;        // tests only: drb_debug_cdae_capture_logits
+  drb_optim_desc opt;  // drb_cdae_set_optimizer (opt_set == false: Adam with the step args' beta1 / beta2 / epsilon)
+  bool opt_set;
   // CUDA-graph replay of the whole step for the launch-bound shapes (ml-100k: ~15 launches of a few microseconds).
   // One instantiated graph per (batch, mask mode, loss pointer, hyper-parameters); it reads the batch from the model's
   // own uids / keep_off / keep buffers and the per-step scalars (five Adam step sizes, philox step) from device memory.
@@ -389,6 +391,8 @@ int drb_cdae_create(drb_ctx* ctx, const drb_cdae_desc* desc, drb_cdae** out) {
   m->ip8 = (int)drb_round_up(L.items_pad, 8);
   m->v_grad_clean = false;
   m->z_dbg = nullptr;
+  std::memset(&m->opt, 0, sizeof(m->opt));
+  m->opt_set = false;
   m->rows_uids = nullptr; m->rows_n = 0; m->reg_slots_clear = false;
   std::memset(m->graphs, 0, sizeof(m->graphs));
   m->n_graphs = m->graph_next = m->n_captures = 0;
@@ -430,6 +434,21 @@ int drb_cdae_create(drb_ctx* ctx, const drb_cdae_desc* desc, drb_cdae** out) {
   *out = m;
   return DRB_OK;
 }
+int drb_cdae_set_optimizer(drb_cdae* m, const drb_optim_desc* opt) {
+  if (!m) return drb_fail(DRB_E_INVALID, "drb_cdae_set_optimizer: NULL model");
+  int r = optim_check(opt, "drb_cdae_set_optimizer");
+  if (r) return r;
+  m->opt = *opt;
+  m->opt_set = true;
+  // captured steps hold the previous rule's kernel and hyper-parameters: never replay them for this one
+  for (int i = 0; i < 8; i++) {
+    if (m->graphs[i].exec) cudaGraphExecDestroy(m->graphs[i].exec);
+    m->graphs[i] = drb_cdae::Graph{};
+  }
+  m->n_graphs = m->graph_next = 0;
+  return DRB_OK;
+}
+
 int drb_cdae_destroy(drb_cdae* m) {
   if (m) {
     for (int i = 0; i < 8; i++)
@@ -501,6 +520,14 @@ int drb_cdae_label_count_buffer(drb_cdae* m, float** ptr, int64_t* count) {
 }
 
 }  // extern "C"
+
+// the optimizer a step runs: the model's descriptor, or Adam with the step args' hyper-parameters when none was set
+static drb_optim_desc effective_optim(bool set, const drb_optim_desc& d, float beta1, float beta2, float eps) {
+  if (set) return d;
+  drb_optim_desc o{};
+  o.kind = DRB_OPT_ADAM; o.beta1 = beta1; o.beta2 = beta2; o.epsilon = eps;
+  return o;
+}
 
 // scal_dev != NULL (graph capture): the five Adam step sizes are read from scal_dev[0..4] (reference variable order
 // [W, W_, V, b, b_]) and the philox step from scal_dev[5..6] (lo, hi words) -- the only per-step scalars of a step
@@ -760,7 +787,9 @@ static int cdae_step_impl(drb_cdae* m, const int32_t* uids, const int32_t* keep_
   //    the V update (72 % of the Adam bytes at the ml-20m shape).
   AdamArgs ad{};
   ad.w = P; ad.m = m->d.adam_m; ad.v = m->d.adam_v; ad.g = G;
-  ad.beta1 = a->beta1; ad.beta2 = a->beta2; ad.eps = a->epsilon;
+  const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, a->beta1, a->beta2, a->epsilon);
+  OptimExtra ox;
+  optim_fill_args(opt, ad, ox);    // update rule, its hyper-parameters and slots (Adam: beta1 / beta2 / eps only)
   ad.alpha_dev = scal_dev;
   const float c = a->reg_rate / (float)gbatch;                      // cdae.py:82
   const int64_t offs[6] = {L.off_w2t, L.off_w, L.off_b, L.off_b2, L.off_v, L.total};   // arena order
@@ -772,7 +801,7 @@ static int cdae_step_impl(drb_cdae* m, const int32_t* uids, const int32_t* keep_
     for (int sidx = first; sidx <= last; sidx++, ns++) {
       ad.seg[ns].off4 = offs[sidx] / 4;
       ad.seg[ns].n4 = (offs[sidx + 1] - offs[sidx]) / 4;
-      ad.seg[ns].alpha = drb_adam_alpha(a->learning_rate, a->beta1, a->beta2, a->t[tmap[sidx]]);
+      ad.seg[ns].alpha = drb_optim_step_size(opt, a->learning_rate, a->t[tmap[sidx]]);
       ad.seg[ns].alpha_idx = tmap[sidx];
       ad.seg[ns].l2 = l2seg[sidx] ? c : 0.f;
       ad.seg[ns].regw = l2seg[sidx] ? 0.5f * c : 0.f;
@@ -784,7 +813,7 @@ static int cdae_step_impl(drb_cdae* m, const int32_t* uids, const int32_t* keep_
       ad.row_mask = w.row_touched; ad.row_seg = 4 - first; ad.row_len4 = ld / 4;
     }
     ad.reg_part = w.reg_part + (int64_t)slot * R;
-    return launch_adam(ctx, ad, n_out);
+    return launch_adam(ctx, ad, n_out, ox);
   };
   auto rezero_user_rows = [&]() -> int {      // leave dV all-zero again for the next step (see PREP)
     if (sharded) return DRB_OK;
@@ -896,7 +925,8 @@ int drb_cdae_step_phases(drb_cdae* m, const int32_t* uids, const int32_t* keep_o
     g = &m->graphs[slot];
   }
   float vals[7];
-  for (int j = 0; j < 5; j++) vals[j] = drb_adam_alpha(a->learning_rate, a->beta1, a->beta2, a->t[j]);
+  const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, a->beta1, a->beta2, a->epsilon);
+  for (int j = 0; j < 5; j++) vals[j] = drb_optim_step_size(opt, a->learning_rate, a->t[j]);
   const uint32_t slo = (uint32_t)a->philox_step, shi = (uint32_t)(a->philox_step >> 32);
   std::memcpy(&vals[5], &slo, 4);
   std::memcpy(&vals[6], &shi, 4);
@@ -1197,6 +1227,8 @@ struct drb_dmf {
   int n_graphs, graph_next, graph_off, n_captures;
   cudaStream_t cap_stream;     // capture happens here (the caller's stream may be the legacy default stream)
   float* step_scalars;
+  drb_optim_desc opt;          // drb_dmf_set_optimizer (opt_set == false: Adam with the step args' hyper-parameters)
+  bool opt_set;
 };
 
 static int dmf_fill_layout(int32_t n_users, int32_t n_items, const int32_t* uf, int32_t nu, const int32_t* itf,
@@ -1375,6 +1407,20 @@ int drb_dmf_create(drb_ctx* ctx, const drb_dmf_desc* d, drb_dmf** out) {
   *out = m;
   return DRB_OK;
 }
+int drb_dmf_set_optimizer(drb_dmf* m, const drb_optim_desc* opt) {
+  if (!m) return drb_fail(DRB_E_INVALID, "drb_dmf_set_optimizer: NULL model");
+  int r = optim_check(opt, "drb_dmf_set_optimizer");
+  if (r) return r;
+  m->opt = *opt;
+  m->opt_set = true;
+  for (int i = 0; i < 8; i++) {     // captured steps hold the previous rule: never replay them for this one
+    if (m->graphs[i].exec) cudaGraphExecDestroy(m->graphs[i].exec);
+    m->graphs[i] = drb_dmf::Graph{};
+  }
+  m->n_graphs = m->graph_next = 0;
+  return DRB_OK;
+}
+
 int drb_dmf_destroy(drb_dmf* m) {
   if (m) {
     for (int i = 0; i < 8; i++)
@@ -1467,11 +1513,13 @@ static int dmf_step_body(drb_dmf* m, const int32_t* uids, const int32_t* iids, c
   if (!(phases & DMF_PHASE_UPDATE)) return DRB_OK;
   AdamArgs ad{};
   ad.w = m->d.params; ad.m = m->d.adam_m; ad.v = m->d.adam_v; ad.g = m->d.grads;
-  ad.beta1 = a->beta1; ad.beta2 = a->beta2; ad.eps = a->epsilon;
+  const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, a->beta1, a->beta2, a->epsilon);
+  OptimExtra ox;
+  optim_fill_args(opt, ad, ox);
   ad.alpha_dev = alpha_dev;
   int ns = 0;
   for (int t = 0; t < 2; t++) {
-    const float alpha = drb_adam_alpha(a->learning_rate, a->beta1, a->beta2, a->t[t]);
+    const float alpha = drb_optim_step_size(opt, a->learning_rate, a->t[t]);
     DmfTower& T = m->tw[t];
     int64_t in = T.in_dim;
     for (int l = 0; l < T.n_layers; l++) {
@@ -1493,7 +1541,7 @@ static int dmf_step_body(drb_dmf* m, const int32_t* uids, const int32_t* iids, c
   ad.fin_n_reg = 0; ad.fin_reg_part = nullptr; ad.fin_loss_out = loss_out;
   ad.fin_ticket = reinterpret_cast<unsigned int*>(m->loss_scalar + 48);
   int n_reg = 0;
-  return launch_adam(ctx, ad, &n_reg);
+  return launch_adam(ctx, ad, &n_reg, ox);
 }
 
 int drb_dmf_step(drb_dmf* m, const int32_t* uids, const int32_t* iids, const float* labels, int32_t batch,
@@ -1573,8 +1621,9 @@ int drb_dmf_step_phases(drb_dmf* m, const int32_t* uids, const int32_t* iids, co
                                      exec, captured};
     g = &m->graphs[slot];
   }
-  const float alphas[2] = {drb_adam_alpha(a->learning_rate, a->beta1, a->beta2, a->t[0]),
-                           drb_adam_alpha(a->learning_rate, a->beta1, a->beta2, a->t[1])};
+  const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, a->beta1, a->beta2, a->epsilon);
+  const float alphas[2] = {drb_optim_step_size(opt, a->learning_rate, a->t[0]),
+                           drb_optim_step_size(opt, a->learning_rate, a->t[1])};
   int r = launch_set_scalars(ctx, m->step_scalars, alphas, 2);
   if (r) return r;
   DRB_CUDA_TRY(ctx, cudaGraphLaunch(g->exec, ctx->stream));

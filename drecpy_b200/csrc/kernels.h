@@ -1,6 +1,6 @@
 // Launcher prototypes of the sm_100a kernels behind libdrb.so (internal, not part of the ABI).
 // Kernel ids follow SURVEY.md section 2b: K1 gather, K2/K3 dense output layer + backward, K3 scatter,
-// K4 fused Adam+L2, K5 DMF head, K6 scoring / top-k.
+// K4 fused optimizer update+L2, K5 DMF head, K6 scoring / top-k.
 #ifndef DRB_KERNELS_H
 #define DRB_KERNELS_H
 
@@ -207,9 +207,25 @@ struct AdamArgs {
   // set in row_mask (the user table of CDAE: only the sampled users' rows): the gradient of the other rows is not read
   const uint32_t* row_mask = nullptr; int row_seg = -1; int row_len4 = 0;
 };
+// the update rule (OPT_*; 0 = Adam) and what only the rules other than Adam read: x = third state arena (AMSGrad vhat,
+// centered RMSprop's momentum), RMSprop's rho, SGD / RMSprop momentum (a kernel argument of its own, so that Adam's
+// kernel keeps its arguments)
+struct OptimExtra { int kind = 0; float* x = nullptr; float momentum = 0.f, rho = 0.f; int nesterov = 0; };
+// update rules of K4, one kernel each (k_adam, k_optim_sgd, ...): the public kind (drb_optim_desc) with the options
+// that change which state arrays are touched resolved at set-up
+enum { OPT_ADAM = 0, OPT_SGD, OPT_SGD_MOMENTUM, OPT_RMSPROP, OPT_RMSPROP_CENTERED, OPT_RMSPROP_MOMENTUM,
+       OPT_RMSPROP_CENTERED_MOMENTUM, OPT_ADAGRAD, OPT_ADAMAX, OPT_AMSGRAD, OPT_N_KINDS };
+const char* optim_kernel_name(int kind);
+int optim_update_kind(const drb_optim_desc& o);                  // -1: not a supported descriptor
+int optim_check(const drb_optim_desc* o, const char* who);       // DRB_OK or DRB_E_INVALID with a message
+void optim_fill_args(const drb_optim_desc& o, AdamArgs& a, OptimExtra& e);   // rule, hyper-parameters, third arena
+// the per-variable step size of segment launches: alpha_t (Adam / AMSGrad), lr_t / (1 - beta1^t) (Adamax), else lr_t;
+// lr_t = lr / (1 + decay (t - 1)), computed in fp32 on the host
+float drb_optim_step_size(const drb_optim_desc& o, float lr, int t);
 // dst[i] = vals[i], i < n <= 8 (one tiny launch; the values travel as kernel arguments)
 int launch_set_scalars(drb_ctx* ctx, float* dst, const float* vals, int n);
-int launch_adam(drb_ctx* ctx, const AdamArgs& a, int* n_blocks_out);
+// the update kernel of a.kind (the launch every UPDATE phase of CDAE and DMF goes through)
+int launch_adam(drb_ctx* ctx, const AdamArgs& a, int* n_blocks_out, const OptimExtra& e = OptimExtra{});
 // loss_out = sum(loss_part) * scale + sum(reg_part)
 int launch_finalize_loss(drb_ctx* ctx, const float* loss_part, int n_loss, float scale, const float* reg_part,
                          int n_reg, float* loss_out);

@@ -21,6 +21,8 @@ _RING = 4
 
 
 class DMF(DeepRecommenderABC):
+    _SET_OPTIMIZER = 'drb_dmf_set_optimizer'
+
     def __init__(self, user_factors=None, item_factors=None, use_nce=True, l2_norm_vectors=True, **kwds):
         super(DMF, self).__init__(**kwds)
         self.user_factors = user_factors
@@ -80,8 +82,7 @@ class DMF(DeepRecommenderABC):
                                       len(self.item_factors), C.byref(L)))
         self._L = L
         self._params = torch.zeros(L.total, dtype=torch.float32, device=self._dev)
-        self._adam_m = torch.zeros_like(self._params)
-        self._adam_v = torch.zeros_like(self._params)
+        self._alloc_optimizer_slots()
         self._grads = torch.zeros_like(self._params)
         gen = torch.Generator().manual_seed(abs(int(self.seed)) if self.seed is not None else random.getrandbits(62))
         for name, factors in (('user_nn', self.user_factors), ('item_nn', self.item_factors)):
@@ -162,6 +163,7 @@ class DMF(DeepRecommenderABC):
         _lib.check(lib.drb_dmf_loss_buffer(self._native, C.byref(ptr)))
         off = ptr.value - self._workspace.data_ptr()
         self._loss_dev = self._workspace[off:off + 8].view(torch.float32)
+        self._apply_optimizer()
 
     def _params_tensor(self):
         return self._params
@@ -170,7 +172,8 @@ class DMF(DeepRecommenderABC):
     def step_args(self, reg_rate):
         o = self.optimizer
         a = _lib.DmfStepArgs()
-        a.learning_rate, a.beta1, a.beta2, a.epsilon = o['learning_rate'], o['beta_1'], o['beta_2'], o['epsilon']
+        a.learning_rate = o['learning_rate']       # the rest of the optimizer is the model's drb_optim_desc
+        a.beta1, a.beta2, a.epsilon = o.get('beta_1', 0.9), o.get('beta_2', 0.999), o.get('epsilon', 1e-7)
         a.reg_rate = reg_rate
         s = self._step
         for g in range(2):

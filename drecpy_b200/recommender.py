@@ -11,6 +11,7 @@ Deliberate, observationally-equivalent change (SURVEY.md Q3): weights are snapsh
 Subclasses implement _pre_fit / _train_step / _predict / _rank_batch on top of libdrb; overriding the math hooks
 with arbitrary framework code is not supported (there is no TensorFlow and no CPU fallback).
 """
+import ctypes as C
 import logging
 import random
 import threading
@@ -18,6 +19,7 @@ from abc import ABC, abstractmethod
 
 import numpy as np
 
+from . import _lib, optimizers
 from .dataset import InteractionData
 from .loss_tracker import LossTracker
 
@@ -64,6 +66,33 @@ class DeepRecommenderABC(ABC):
     # ------------------------------------------------------------------ fit (recommender_abc.py:97-264)
     def fit(self, interaction_dataset, epochs=50, batch_size=32, learning_rate=0.001, neg_ratio=5, reg_rate=0.001,
             copy_dataset=False, **kwds):
+        """Trains the model as the reference's fit() does (same keywords, callbacks, early stopping and reverts).
+
+        optimizer=: None (Keras Adam with `learning_rate`), a dict without 'name' (overrides of that Adam: learning_rate,
+        beta_1, beta_2, epsilon, amsgrad, decay; any other key raises ValueError), a dict with 'name', or a tf.keras optimizer (read through its
+        get_config(); TensorFlow is not imported).  An explicit optimizer carries its own learning rate (a named dict
+        without one takes the Keras default); `learning_rate` only builds the default Adam.  Supported, with the Keras-2 /
+        TF 2.0-2.3 dense updates in fp32 (g = gradient + L2 term; every element updated every step; slots start at 0):
+          SGD(0.01, momentum=0, nesterov=False)   momentum 0: w -= lr*g; else a = a*momentum - lr*g, then w += a, or
+                                                  with nesterov w += a*momentum - lr*g
+          RMSprop(0.001, rho=0.9, momentum=0, epsilon=1e-7, centered=False)
+                                                  momentum 0: ms = rho*ms + (1-rho)*g^2; centered: mg = rho*mg +
+                                                  (1-rho)*g, d = ms - mg^2, else d = ms; w -= lr*g / (sqrt(d) + eps).
+                                                  momentum > 0: ms += (g^2 - ms)*(1-rho); centered: mg += (g - mg)*(1-rho),
+                                                  d = ms - mg^2 + eps, else d = ms + eps; mom = mom*momentum +
+                                                  lr*g / sqrt(d); w -= mom
+          Adagrad(0.001, initial_accumulator_value=0.1, epsilon=1e-7)
+                                                  acc (starts at initial_accumulator_value) += g^2;
+                                                  w -= lr*g / (sqrt(acc) + eps)
+          Adamax(0.001, beta_1=0.9, beta_2=0.999, epsilon=1e-7)
+                                                  m += (g - m)*(1-beta_1); u = max(beta_2*u, |g|);
+                                                  w -= lr/(1 - beta_1^t) * m/(u + eps)
+          Adam(0.001, beta_1=0.9, beta_2=0.999, epsilon=1e-7, amsgrad=False)
+                                                  Keras Adam; amsgrad: vhat = max(vhat, v), w -= alpha_t*m/(sqrt(vhat)+eps)
+        t is the per-variable step counter (adam_t); Keras-2 `decay` gives lr_t = lr / (1 + decay*(t - 1)), applied
+        before any bias correction.  Learning-rate schedules, clipnorm / clipvalue / global_clipnorm and other
+        optimizers (Nadam, Ftrl, Adadelta, ...) raise NotImplementedError.  Weight snapshots and reverts restore the
+        weights only, not the optimizer's slots."""
         self.interaction_dataset = interaction_dataset
         if copy_dataset and hasattr(interaction_dataset, '__copy__'):
             self._info('Cloning new dataset instance...')
@@ -83,13 +112,7 @@ class DeepRecommenderABC(ABC):
         self._log_initial_info()
         self._info('Creating auxiliary structures...')
 
-        opt = kwds.get('optimizer', None)
-        if opt is not None and not isinstance(opt, dict):
-            raise NotImplementedError('drecpy_b200 runs Keras-Adam natively; pass optimizer=None or a dict with '
-                                      'beta_1 / beta_2 / epsilon / learning_rate overrides')
-        self.optimizer = {'learning_rate': learning_rate, 'beta_1': 0.9, 'beta_2': 0.999, 'epsilon': 1e-7}
-        if opt:
-            self.optimizer.update(opt)
+        self.optimizer = optimizers.parse(kwds.get('optimizer', None), learning_rate)
         self._step = 0
         self.epoch_weights = {}
         self._pre_fit(learning_rate, neg_ratio, reg_rate, batch_size=batch_size, **kwds)
@@ -190,6 +213,23 @@ class DeepRecommenderABC(ABC):
 
     def _finish_fit(self):
         pass
+
+    # ------------------------------------------------------------------ optimizer slots (adam_m / adam_v / third arena)
+    _SET_OPTIMIZER = None        # name of the drb_*_set_optimizer entry point of the subclass
+
+    def _alloc_optimizer_slots(self):
+        """The optimizer's slot arenas, shaped like the parameter arena: adam_m (Adagrad: initial_accumulator_value),
+        adam_v, and the third arena only for AMSGrad and centered RMSprop with momentum."""
+        torch = self._torch
+        self._adam_m = torch.full_like(self._params, optimizers.initial_m(self.optimizer))
+        self._adam_v = torch.zeros_like(self._params)
+        self._optim_x = torch.zeros_like(self._params) if optimizers.needs_third_state(self.optimizer) else None
+
+    def _apply_optimizer(self):
+        """Hands self.optimizer and its slots to the native model (every step after this call runs that update)."""
+        x = getattr(self, '_optim_x', None)
+        desc = optimizers.native_desc(self.optimizer, x.data_ptr() if x is not None else None)
+        _lib.check(getattr(_lib.load(), self._SET_OPTIMIZER)(self._native, C.byref(desc)))
 
     def _params_tensor(self):
         raise NotImplementedError
@@ -465,8 +505,8 @@ class DeepRecommenderABC(ABC):
     def __getstate__(self):
         """joblib/pickle: device arenas go to host tensors, native handles are dropped and rebuilt on load."""
         st = {k: v for k, v in self.__dict__.items() if k not in self._TRANSIENT}
-        for k in ('_params', '_adam_m', '_adam_v', '_grads'):
-            if k in st: st[k] = st[k].cpu()
+        for k in ('_params', '_adam_m', '_adam_v', '_grads', '_optim_x'):
+            if st.get(k) is not None: st[k] = st[k].cpu()
         L = getattr(self, '_L', None)
         st['_L'] = (type(L), {f: (list(getattr(L, f)) if hasattr(getattr(L, f), '__len__') else getattr(L, f))
                               for f, _ in L._fields_}) if L is not None else None
@@ -493,8 +533,9 @@ class DeepRecommenderABC(ABC):
                     setattr(self._L, f, v)
             self._dp = DataParallel()
             self._dev = torch.device(self.device or f'cuda:{torch.cuda.current_device()}')
-            for k in ('_params', '_adam_m', '_adam_v', '_grads'):
-                setattr(self, k, getattr(self, k).to(self._dev))
+            for k in ('_params', '_adam_m', '_adam_v', '_grads', '_optim_x'):
+                if getattr(self, k, None) is not None:
+                    setattr(self, k, getattr(self, k).to(self._dev))
             self._build_native()
 
     def save(self, save_path):

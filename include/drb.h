@@ -201,6 +201,39 @@ typedef struct {
                               launch-bound small shapes replay the step as a CUDA graph from device-resident inputs */
 } drb_cdae_step_args;
 
+/* ------------------------------------------------------------------ optimizer of the dense update (K4)
+ * replaces: the `optimizer=` keyword of recommender_abc.py:153 (any tf.keras optimizer, applied per variable at
+ * :328-334).  Keras-2 / TF 2.0-2.3 OptimizerV2 dense updates in fp32; g is the gradient with the L2 term folded in:
+ *   DRB_OPT_SGD      momentum == 0: w -= lr_t g;  else a = a momentum - lr_t g (slot adam_m), w += a, or with
+ *                    nesterov w += a momentum - lr_t g
+ *   DRB_OPT_RMSPROP  momentum == 0: ms = rho ms + (1-rho) g^2 (adam_m); centered: mg = rho mg + (1-rho) g (adam_v),
+ *                    d = ms - mg^2, else d = ms; w -= lr_t g / (sqrt(d) + eps).
+ *                    momentum > 0: ms += (g^2 - ms)(1-rho); centered: mg += (g - mg)(1-rho), d = ms - mg^2 + eps, else
+ *                    d = ms + eps; mom = mom momentum + lr_t g / sqrt(d) (adam_v, or third_state when centered); w -= mom
+ *   DRB_OPT_ADAGRAD  acc += g^2 (adam_m, which the caller initialises to initial_accumulator_value);
+ *                    w -= lr_t g / (sqrt(acc) + eps)
+ *   DRB_OPT_ADAMAX   m += (g - m)(1-beta1); u = max(beta2 u, |g|) (adam_v); w -= lr_t / (1 - beta1^t) m / (u + eps)
+ *   DRB_OPT_ADAM     Keras Adam; amsgrad != 0: vhat = max(vhat, v) (third_state), w -= alpha_t m / (sqrt(vhat) + eps)
+ * lr_t = learning_rate / (1 + decay (t - 1)) with learning_rate and the per-variable counters t of the step args.
+ * A model that never calls drb_*_set_optimizer runs Adam with the beta1 / beta2 / epsilon of its step args; once it is
+ * called, the descriptor's values are used instead (the step args then supply learning_rate and t only).  The slots are
+ * the model's adam_m / adam_v arenas and, for AMSGrad and centered RMSprop with momentum only, third_state: a device
+ * arena of the parameter arena's size and layout (caller-owned, 16-byte aligned, zero-initialised), borrowed until the
+ * next call or the model's destruction.  Setting an optimizer does not touch any arena. */
+enum { DRB_OPT_ADAM = 0, DRB_OPT_SGD = 1, DRB_OPT_RMSPROP = 2, DRB_OPT_ADAGRAD = 3, DRB_OPT_ADAMAX = 4 };
+typedef struct {
+  int32_t kind;            /* DRB_OPT_* */
+  float momentum;          /* SGD, RMSprop: >= 0 */
+  int32_t nesterov;        /* SGD */
+  float rho;               /* RMSprop */
+  int32_t centered;        /* RMSprop */
+  float beta1, beta2;      /* Adam, Adamax: in [0, 1) */
+  float epsilon;           /* > 0 for RMSprop, Adagrad, Adamax */
+  int32_t amsgrad;         /* Adam */
+  float decay;             /* Keras-2 time decay of the learning rate, >= 0 */
+  float* third_state;      /* AMSGrad vhat / centered RMSprop with momentum: its momentum; else ignored (may be NULL) */
+} drb_optim_desc;
+
 enum {
   DRB_PHASE_PREP = 1,      /* clear gradients, label histogram / bitmap, philox mask */
   DRB_PHASE_GRADS_A = 2,   /* hidden layer (gather) + tf32 operand splits: needs no labels */
@@ -225,6 +258,9 @@ enum {
 
 int drb_cdae_create(drb_ctx* ctx, const drb_cdae_desc* desc, drb_cdae** out);
 int drb_cdae_destroy(drb_cdae* m);
+/* Selects the optimizer of every following step (see drb_optim_desc).  DRB_E_INVALID with a message for a descriptor
+ * out of range.  Graphs captured for the previous optimizer are dropped. */
+int drb_cdae_set_optimizer(drb_cdae* m, const drb_optim_desc* opt);
 /* One training step on device-resident inputs.
  * replaces: recommender_abc.py:190-205 (tape, gradient, 5x apply_gradients) with cdae.py:50-82 inside.
  * uids[batch], keep_off[batch+1], keep[keep_off[batch]] are DEVICE pointers; keep == NULL selects the
@@ -330,6 +366,8 @@ typedef struct {
 
 int drb_dmf_create(drb_ctx* ctx, const drb_dmf_desc* desc, drb_dmf** out);
 int drb_dmf_destroy(drb_dmf* m);
+/* drb_cdae_set_optimizer for DMF (t of the step args: the per-tower counters) */
+int drb_dmf_set_optimizer(drb_dmf* m, const drb_optim_desc* opt);
 /* replaces: recommender_abc.py:190-205 with dmf.py:64-99 inside.  uids/iids/labels: device [batch];
  * loss_out: device float[2] ([0] reported loss, [1] its batch term). */
 int drb_dmf_step(drb_dmf* m, const int32_t* uids, const int32_t* iids, const float* labels, int32_t batch,
