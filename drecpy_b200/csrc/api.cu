@@ -201,6 +201,91 @@ int drb_debug_umma_gemm_f16(drb_ctx* ctx, const void* a_hi, const void* a_lo, in
 
 }  // extern "C"
 
+// ========================================================================================== step graphs
+// CUDA-graph replay of a training step for the launch-bound shapes (a few microseconds per kernel).  One instantiated
+// graph per argument set: the captured step reads its batch from the model's own buffers and its per-step scalars
+// from device memory, which a one-thread kernel (k_set_scalars) refreshes before every replay.
+struct StepGraphKey {   // a model fills the fields its step depends on and leaves the others zero
+  const void* loss_out; int32_t batch, phases, global_batch, has_keep;
+  float beta1, beta2, eps, reg; uint64_t philox_seed;
+  bool operator==(const StepGraphKey& o) const {   // field by field: a NaN hyper-parameter never matches
+    return loss_out == o.loss_out && batch == o.batch && phases == o.phases && global_batch == o.global_batch &&
+           has_keep == o.has_keep && beta1 == o.beta1 && beta2 == o.beta2 && eps == o.eps && reg == o.reg &&
+           philox_seed == o.philox_seed;
+  }
+};
+
+struct StepGraphs {
+  struct Entry { StepGraphKey key; cudaGraphExec_t exec; int64_t launches; };
+  static constexpr int kSlots = 8;          // live graphs; beyond that a capture replaces one, round robin
+  static constexpr int kMaxCaptures = 32;   // a caller that keeps changing the argument set would pay a capture per step
+  Entry slots[kSlots];                      // [0, n_live) hold live execs
+  int n_live = 0, next = 0, n_captures = 0;
+  bool off;                                 // direct launches: DRB_GRAPH=0, or graphs were given up
+  cudaStream_t stream = nullptr;            // capture happens here (the caller's stream may be the legacy default stream)
+
+  StepGraphs() { const char* ge = getenv("DRB_GRAPH"); off = ge && atoi(ge) == 0; }
+  StepGraphs(const StepGraphs&) = delete;   // owns the execs and the stream
+  StepGraphs& operator=(const StepGraphs&) = delete;
+  ~StepGraphs() {
+    clear();
+    if (stream) cudaStreamDestroy(stream);
+  }
+
+  // The entry for `key`.  On a miss `body()` (the step, enqueued on ctx->stream) is captured: nothing executes and its
+  // launches are not counted.  nullptr: graphs are off -- from now on if the capture failed or too many were taken --
+  // and the caller launches the step directly.
+  template <class Body>
+  Entry* get(drb_ctx* ctx, const StepGraphKey& key, Body&& body) {
+    if (off) return nullptr;
+    for (int i = 0; i < n_live; i++)
+      if (slots[i].key == key) return &slots[i];
+    if (++n_captures <= kMaxCaptures &&
+        (stream || cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking) == cudaSuccess)) {
+      cudaStream_t user = ctx->stream;
+      const int64_t before = ctx->launches;
+      cudaGraph_t graph = nullptr;
+      cudaGraphExec_t exec = nullptr;
+      int r = DRB_OK;
+      cudaError_t e = cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal);
+      if (e == cudaSuccess) {
+        ctx->stream = stream;
+        r = body();
+        ctx->stream = user;
+        e = cudaStreamEndCapture(stream, &graph);
+      }
+      if (e == cudaSuccess && r == DRB_OK) e = cudaGraphInstantiate(&exec, graph, 0);
+      if (graph) cudaGraphDestroy(graph);
+      const int64_t captured = ctx->launches - before;
+      ctx->launches = before;
+      if (e == cudaSuccess && r == DRB_OK) {
+        if (n_live == kSlots) cudaGraphExecDestroy(slots[next % kSlots].exec);
+        Entry& s = slots[n_live < kSlots ? n_live++ : next++ % kSlots];
+        s = Entry{key, exec, captured};
+        return &s;
+      }
+    }
+    cudaGetLastError();   // e.g. a driver without capture support for some node, or too many captures
+    ctx->sticky = 0;
+    off = true;
+    return nullptr;
+  }
+
+  // refresh the n per-step scalars at scal_dev, then replay; counts k_set_scalars and the captured launches
+  int replay(drb_ctx* ctx, const Entry* g, float* scal_dev, const float* vals, int n) {
+    int r = launch_set_scalars(ctx, scal_dev, vals, n);
+    if (r) return r;
+    DRB_CUDA_TRY(ctx, cudaGraphLaunch(g->exec, ctx->stream));
+    ctx->launches += g->launches;
+    return DRB_OK;
+  }
+
+  void clear() {   // drops every graph; the capture count stays
+    for (int i = 0; i < n_live; i++) cudaGraphExecDestroy(slots[i].exec);
+    n_live = next = 0;
+  }
+};
+
 // ========================================================================================== CDAE
 struct CdaeWs {
   float *h, *dz, *dh_part, *dz1, *col_b2, *col_b, *loss_part, *reg_part, *label_count, *loss_scalar;
@@ -232,15 +317,9 @@ struct drb_cdae {
   float* z_dbg;        // tests only: drb_debug_cdae_capture_logits
   drb_optim_desc opt;  // drb_cdae_set_optimizer (opt_set == false: Adam with the step args' beta1 / beta2 / epsilon)
   bool opt_set;
-  // CUDA-graph replay of the whole step for the launch-bound shapes (ml-100k: ~15 launches of a few microseconds).
-  // One instantiated graph per (batch, mask mode, loss pointer, hyper-parameters); it reads the batch from the model's
-  // own uids / keep_off / keep buffers and the per-step scalars (five Adam step sizes, philox step) from device memory.
-  struct Graph {
-    const void* loss_out; int32_t batch; int has_keep; float beta1, beta2, eps, reg, lr_unused;
-    uint64_t philox_seed; cudaGraphExec_t exec; int64_t launches;
-  } graphs[8];
-  int n_graphs, graph_next, graph_off, n_captures;
-  cudaStream_t cap_stream;
+  // the whole step of the launch-bound shapes (ml-100k: ~15 launches) replayed from the uids / keep_off / keep
+  // buffers above, with the five Adam step sizes and the philox step at ws.loss_scalar + 8
+  StepGraphs graphs;
 };
 
 // N of the backward GEMMs: hidden plus the constant-one feature that folds db' = colsum(dz) into dW'^T, rounded to 16.
@@ -394,10 +473,6 @@ int drb_cdae_create(drb_ctx* ctx, const drb_cdae_desc* desc, drb_cdae** out) {
   std::memset(&m->opt, 0, sizeof(m->opt));
   m->opt_set = false;
   m->rows_uids = nullptr; m->rows_n = 0; m->reg_slots_clear = false;
-  std::memset(m->graphs, 0, sizeof(m->graphs));
-  m->n_graphs = m->graph_next = m->n_captures = 0;
-  m->cap_stream = nullptr;
-  { const char* ge = getenv("DRB_GRAPH"); m->graph_off = (ge && atoi(ge) == 0) ? 1 : 0; }   // DRB_GRAPH=0: direct launches
   if (m->use_umma) {
     // dh = dz W'^T on the tensor cores has one 128 x n2 tile per 128 users: split the item range so that the grid
     // is ~2 waves of the SM count (the kernel is L2/HBM bandwidth bound, one CTA per SM)
@@ -440,21 +515,11 @@ int drb_cdae_set_optimizer(drb_cdae* m, const drb_optim_desc* opt) {
   if (r) return r;
   m->opt = *opt;
   m->opt_set = true;
-  // captured steps hold the previous rule's kernel and hyper-parameters: never replay them for this one
-  for (int i = 0; i < 8; i++) {
-    if (m->graphs[i].exec) cudaGraphExecDestroy(m->graphs[i].exec);
-    m->graphs[i] = drb_cdae::Graph{};
-  }
-  m->n_graphs = m->graph_next = 0;
+  m->graphs.clear();   // captured steps hold the previous rule's kernel and hyper-parameters: never replay them for this one
   return DRB_OK;
 }
 
 int drb_cdae_destroy(drb_cdae* m) {
-  if (m) {
-    for (int i = 0; i < 8; i++)
-      if (m->graphs[i].exec) cudaGraphExecDestroy(m->graphs[i].exec);
-    if (m->cap_stream) cudaStreamDestroy(m->cap_stream);
-  }
   delete m;
   return DRB_OK;
 }
@@ -865,7 +930,7 @@ int drb_cdae_step_phases(drb_cdae* m, const int32_t* uids, const int32_t* keep_o
   // captured step is the sparse-clear variant), with inputs that can be staged in the model's own buffers.
   const bool own_inputs = uids == m->ws.uids && keep_off == m->ws.keep_off && (!keep || keep == m->ws.keep);
   const bool small = (int64_t)batch * m->d.n_items <= ((int64_t)8 << 20);
-  const bool eligible = !m->graph_off && !ctx->profile && small && phases == DRB_PHASE_ALL && m->v_grad_clean &&
+  const bool eligible = !m->graphs.off && !ctx->profile && small && phases == DRB_PHASE_ALL && m->v_grad_clean &&
                         a->global_batch == 0 && !a->shard_items && !a->skip_user_grad && !m->z_dbg &&
                         batch > 0 && batch <= m->d.max_batch && m->d.adam_m && !ctx->sticky &&
                         (own_inputs || !keep || a->keep_bytes > 0);
@@ -880,60 +945,23 @@ int drb_cdae_step_phases(drb_cdae* m, const int32_t* uids, const int32_t* keep_o
       DRB_CUDA_TRY(ctx, cudaMemcpyAsync(w.keep, keep, (size_t)a->keep_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
   }
   const uint8_t* gkeep = keep ? w.keep : nullptr;
-  drb_cdae::Graph* g = nullptr;
-  for (int i = 0; i < m->n_graphs; i++) {
-    drb_cdae::Graph& c = m->graphs[i];
-    if (c.loss_out == loss_out && c.batch == batch && c.has_keep == (keep ? 1 : 0) && c.beta1 == a->beta1 &&
-        c.beta2 == a->beta2 && c.eps == a->epsilon && c.reg == a->reg_rate && c.philox_seed == a->philox_seed) { g = &c; break; }
-  }
   float* scal = w.loss_scalar + 8;      // [8..14]: five step sizes + philox step (lo, hi)
-  if (!g) {
-    if (++m->n_captures > 32 ||
-        (!m->cap_stream && cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking) != cudaSuccess)) {
-      cudaGetLastError();
-      m->graph_off = 1;
-      return cdae_step_impl(m, w.uids, w.keep_off, gkeep, batch, a, loss_out, phases, nullptr);
-    }
-    cudaStream_t user = ctx->stream;
-    const int64_t before = ctx->launches;
+  const StepGraphKey key{loss_out, batch, 0, 0, keep ? 1 : 0, a->beta1, a->beta2, a->epsilon, a->reg_rate, a->philox_seed};
+  const StepGraphs::Entry* g = m->graphs.get(ctx, key, [&] {
     const bool clean_before = m->v_grad_clean;
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
-    int r = DRB_OK;
-    cudaError_t e = cudaStreamBeginCapture(m->cap_stream, cudaStreamCaptureModeThreadLocal);
-    if (e == cudaSuccess) {
-      ctx->stream = m->cap_stream;
-      r = cdae_step_impl(m, w.uids, w.keep_off, gkeep, batch, a, loss_out, phases, scal);
-      ctx->stream = user;
-      e = cudaStreamEndCapture(m->cap_stream, &graph);
-    }
-    if (e == cudaSuccess && r == DRB_OK) e = cudaGraphInstantiate(&exec, graph, 0);
-    if (graph) cudaGraphDestroy(graph);
-    const int64_t captured = ctx->launches - before;
-    ctx->launches = before;
+    int r = cdae_step_impl(m, w.uids, w.keep_off, gkeep, batch, a, loss_out, phases, scal);
     m->v_grad_clean = clean_before;      // nothing ran during capture
-    if (e != cudaSuccess || r != DRB_OK) {
-      cudaGetLastError();
-      ctx->sticky = 0;
-      m->graph_off = 1;
-      return cdae_step_impl(m, w.uids, w.keep_off, gkeep, batch, a, loss_out, phases, nullptr);
-    }
-    const int slot = m->n_graphs < 8 ? m->n_graphs++ : (m->graph_next++ & 7);
-    if (m->graphs[slot].exec) cudaGraphExecDestroy(m->graphs[slot].exec);
-    m->graphs[slot] = drb_cdae::Graph{loss_out, batch, keep ? 1 : 0, a->beta1, a->beta2, a->epsilon, a->reg_rate, 0.f,
-                                      a->philox_seed, exec, captured};
-    g = &m->graphs[slot];
-  }
+    return r;
+  });
+  if (!g) return cdae_step_impl(m, w.uids, w.keep_off, gkeep, batch, a, loss_out, phases, nullptr);
   float vals[7];
   const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, a->beta1, a->beta2, a->epsilon);
   for (int j = 0; j < 5; j++) vals[j] = drb_optim_step_size(opt, a->learning_rate, a->t[j]);
   const uint32_t slo = (uint32_t)a->philox_step, shi = (uint32_t)(a->philox_step >> 32);
   std::memcpy(&vals[5], &slo, 4);
   std::memcpy(&vals[6], &shi, 4);
-  int r = launch_set_scalars(ctx, scal, vals, 7);
+  int r = m->graphs.replay(ctx, g, scal, vals, 7);
   if (r) return r;
-  DRB_CUDA_TRY(ctx, cudaGraphLaunch(g->exec, ctx->stream));
-  ctx->launches += g->launches;
   m->v_grad_clean = true;      // the captured step ends with the sparse re-zero of the sampled users' rows
   m->rows_uids = nullptr; m->rows_n = 0;
   return DRB_OK;
@@ -1214,18 +1242,9 @@ struct drb_dmf {
   void* rank_scratch; int64_t rank_scratch_bytes;   // sort keys of candidate lists longer than 4096 (score.cu)
   bool item_rep_valid;                               // item_rep holds the item tower of the CURRENT weights
   int64_t ws_bytes;
-  // CUDA-graph replay of the training step (the C2 step is ~20 launches of a few microseconds each: launch bound).
-  // One instantiated graph per distinct argument set; the Adam step sizes -- the only per-step scalars -- are read
-  // from step_scalars, which a one-thread kernel refreshes before every replay.
-  // The graph always reads the batch from the model's own uids / iids / labels buffers (a caller's device arrays are
-  // copied there first), so there is one graph per (batch size, loss pointer, hyper-parameters).
-  struct Graph {
-    const void* loss_out;
-    int32_t batch, phases, global_batch; float beta1, beta2, eps, reg;
-    cudaGraphExec_t exec; int64_t launches;
-  } graphs[8];
-  int n_graphs, graph_next, graph_off, n_captures;
-  cudaStream_t cap_stream;     // capture happens here (the caller's stream may be the legacy default stream)
+  // the training step replayed from the uids / iids / labels buffers above (a caller's device arrays are copied there
+  // first), with the two Adam step sizes -- the only per-step scalars -- at step_scalars
+  StepGraphs graphs;
   float* step_scalars;
   drb_optim_desc opt;          // drb_dmf_set_optimizer (opt_set == false: Adam with the step args' hyper-parameters)
   bool opt_set;
@@ -1373,11 +1392,9 @@ int drb_dmf_create(drb_ctx* ctx, const drb_dmf_desc* d, drb_dmf** out) {
   if (((uintptr_t)d->params | (uintptr_t)d->adam_m | (uintptr_t)d->adam_v | (uintptr_t)d->grads |
        (uintptr_t)d->workspace) & 15)
     return drb_fail(DRB_E_INVALID, "drb_dmf_create: arenas and workspace must be 16-byte aligned");
-  drb_dmf* m = new (std::nothrow) drb_dmf;
+  drb_dmf* m = new (std::nothrow) drb_dmf();
   if (!m) return drb_fail(DRB_E_NOMEM, "out of memory");
-  std::memset(m, 0, sizeof(*m));
   m->ctx = ctx; m->d = *d; m->L = L;
-  { const char* ge = getenv("DRB_GRAPH"); m->graph_off = (ge && atoi(ge) == 0) ? 1 : 0; }   // DRB_GRAPH=0: direct launches
   for (int t = 0; t < 2; t++) {
     DmfTower& T = m->tw[t];
     T.n_layers = t ? L.n_layers_item : L.n_layers_user;
@@ -1413,20 +1430,11 @@ int drb_dmf_set_optimizer(drb_dmf* m, const drb_optim_desc* opt) {
   if (r) return r;
   m->opt = *opt;
   m->opt_set = true;
-  for (int i = 0; i < 8; i++) {     // captured steps hold the previous rule: never replay them for this one
-    if (m->graphs[i].exec) cudaGraphExecDestroy(m->graphs[i].exec);
-    m->graphs[i] = drb_dmf::Graph{};
-  }
-  m->n_graphs = m->graph_next = 0;
+  m->graphs.clear();   // captured steps hold the previous rule: never replay them for this one
   return DRB_OK;
 }
 
 int drb_dmf_destroy(drb_dmf* m) {
-  if (m) {
-    for (int i = 0; i < 8; i++)
-      if (m->graphs[i].exec) cudaGraphExecDestroy(m->graphs[i].exec);
-    if (m->cap_stream) cudaStreamDestroy(m->cap_stream);
-  }
   delete m;
   return DRB_OK;
 }
@@ -1568,67 +1576,22 @@ int drb_dmf_step_phases(drb_dmf* m, const int32_t* uids, const int32_t* iids, co
   drb_ctx* ctx = m->ctx;
   if (ctx->sticky) return drb_fail(DRB_E_CUDA, "context has a sticky CUDA error (%d)", ctx->sticky);
   m->item_rep_valid = false;           // the weights are about to change
-  if (m->graph_off || ctx->profile)    // per-kernel profiling brackets every launch with events: direct launches
+  if (m->graphs.off || ctx->profile)    // per-kernel profiling brackets every launch with events: direct launches
     return dmf_step_body(m, uids, iids, labels, batch, a, loss_out, nullptr, phases, global_batch);
 
   if (uids != m->uids) DRB_CUDA_TRY(ctx, cudaMemcpyAsync(m->uids, uids, (size_t)batch * 4, cudaMemcpyDeviceToDevice, ctx->stream));
   if (iids != m->iids) DRB_CUDA_TRY(ctx, cudaMemcpyAsync(m->iids, iids, (size_t)batch * 4, cudaMemcpyDeviceToDevice, ctx->stream));
   if (labels != m->labels)
     DRB_CUDA_TRY(ctx, cudaMemcpyAsync(m->labels, labels, (size_t)batch * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-  drb_dmf::Graph* g = nullptr;
-  for (int i = 0; i < m->n_graphs; i++) {
-    drb_dmf::Graph& c = m->graphs[i];
-    if (c.loss_out == loss_out && c.batch == batch && c.phases == phases && c.global_batch == global_batch &&
-        c.beta1 == a->beta1 && c.beta2 == a->beta2 && c.eps == a->epsilon && c.reg == a->reg_rate) { g = &c; break; }
-  }
-  if (!g) {
-    // capture the step once for this argument set (nothing executes during capture); a caller that keeps changing
-    // the argument set would pay a capture per step: give up on graphs after 32 captures
-    if (++m->n_captures > 32) {
-      m->graph_off = 1;
-      return dmf_step_body(m, m->uids, m->iids, m->labels, batch, a, loss_out, nullptr, phases, global_batch);
-    }
-    if (!m->cap_stream && cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking) != cudaSuccess) {
-      cudaGetLastError();
-      m->graph_off = 1;
-      return dmf_step_body(m, uids, iids, labels, batch, a, loss_out, nullptr, phases, global_batch);
-    }
-    cudaStream_t user = ctx->stream;
-    const int64_t before = ctx->launches;
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
-    int r = DRB_OK;
-    cudaError_t e = cudaStreamBeginCapture(m->cap_stream, cudaStreamCaptureModeThreadLocal);
-    if (e == cudaSuccess) {
-      ctx->stream = m->cap_stream;
-      r = dmf_step_body(m, m->uids, m->iids, m->labels, batch, a, loss_out, m->step_scalars, phases, global_batch);
-      ctx->stream = user;
-      e = cudaStreamEndCapture(m->cap_stream, &graph);
-    }
-    if (e == cudaSuccess && r == DRB_OK) e = cudaGraphInstantiate(&exec, graph, 0);
-    if (graph) cudaGraphDestroy(graph);
-    const int64_t captured = ctx->launches - before;
-    ctx->launches = before;
-    if (e != cudaSuccess || r != DRB_OK) {   // e.g. a driver without capture support for some node: run directly from now on
-      cudaGetLastError();
-      ctx->sticky = 0;
-      m->graph_off = 1;
-      return dmf_step_body(m, uids, iids, labels, batch, a, loss_out, nullptr, phases, global_batch);
-    }
-    const int slot = m->n_graphs < 8 ? m->n_graphs++ : (m->graph_next++ & 7);
-    if (m->graphs[slot].exec) cudaGraphExecDestroy(m->graphs[slot].exec);
-    m->graphs[slot] = drb_dmf::Graph{loss_out, batch, phases, global_batch, a->beta1, a->beta2, a->epsilon, a->reg_rate,
-                                     exec, captured};
-    g = &m->graphs[slot];
-  }
+  const StepGraphKey key{loss_out, batch, phases, global_batch, 0, a->beta1, a->beta2, a->epsilon, a->reg_rate, 0};
+  const StepGraphs::Entry* g = m->graphs.get(ctx, key, [&] {
+    return dmf_step_body(m, m->uids, m->iids, m->labels, batch, a, loss_out, m->step_scalars, phases, global_batch);
+  });
+  if (!g) return dmf_step_body(m, m->uids, m->iids, m->labels, batch, a, loss_out, nullptr, phases, global_batch);
   const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, a->beta1, a->beta2, a->epsilon);
   const float alphas[2] = {drb_optim_step_size(opt, a->learning_rate, a->t[0]),
                            drb_optim_step_size(opt, a->learning_rate, a->t[1])};
-  int r = launch_set_scalars(ctx, m->step_scalars, alphas, 2);
-  if (r) return r;
-  DRB_CUDA_TRY(ctx, cudaGraphLaunch(g->exec, ctx->stream));
-  ctx->launches += g->launches;
-  return DRB_OK;
+  return m->graphs.replay(ctx, g, m->step_scalars, alphas, 2);
 }
 
 int drb_dmf_loss_buffer(drb_dmf* m, float** ptr) {

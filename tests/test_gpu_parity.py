@@ -298,6 +298,44 @@ def test_cdae_graph_replay_equals_direct_launches(monkeypatch, mask):
     assert np.max(np.abs(l - lo) / np.abs(lo)) < 1e-3
 
 
+@pytest.mark.parametrize('model', ['cdae', 'dmf'])
+def test_graph_capture_cap_and_slot_replacement(monkeypatch, model):
+    """How a model keeps its step graphs.  Cap: a new reg_rate every step is a new argument set every step, so every
+    step is a capture; after 32 captures the model gives up on graphs and launches directly.  Replacement: ten batch
+    sizes, cycled twice, through the eight graph slots.  Either way graph mode computes what direct launches compute
+    and adds one k_set_scalars launch per replayed step (CDAE's first step runs directly: dV is not yet known clean)."""
+    U, I = 300, 500
+    ds = _dataset(U, I, 15000, seed=8)
+    if model == 'cdae':
+        B, reg, w = 48, 1e-3, _cdae_weights(U, I, 24)
+    else:
+        B, reg, w = 64, 1e-4, _dmf_weights(U, I, [64, 32], [64, 32])
+
+    def make():
+        if model == 'cdae':
+            return _make_cdae(ds, 24, B, w)
+        m = drb.DMF(user_factors=[64, 32], item_factors=[64, 32], seed=10, verbose=False)
+        m.fit(ds, epochs=0, batch_size=B, learning_rate=1e-3, neg_ratio=5, reg_rate=reg, init_weights=w)
+        return m
+    first_direct = 1 if model == 'cdae' else 0
+    cap = [(B, reg * (1 + s / 64)) for s in range(40)]
+    cycle = [(B - 4 * j, reg) for j in range(10)] * 2
+    for steps, replayed in ((cap, 32), (cycle, len(cycle) - first_direct)):
+        runs = []
+        for graph in ('1', '0'):
+            monkeypatch.setenv('DRB_GRAPH', graph)
+            m = make()
+            n0 = m.launch_count()
+            losses = []
+            for s, (b, r) in enumerate(steps, 1):
+                m._step = s
+                losses.append(m._train_step(b, r, want_loss=True))
+            runs.append((losses, m.launch_count() - n0, m._params.cpu().numpy()))
+        assert np.allclose(runs[0][0], runs[1][0], rtol=2e-6, atol=0), (runs[0][0], runs[1][0])
+        assert runs[0][1] == runs[1][1] + replayed
+        assert rel_err(runs[0][2], runs[1][2]) < 1e-5
+
+
 @pytest.mark.parametrize('loss,K', [('bce', 36), ('mse', 200)])
 def test_cdae_sampled_output_steps_vs_oracle(loss, K):
     """The sampled-output extension (BASELINE configs[4]'s mode): positives + 2 groups x 20 drawn items per sampled
