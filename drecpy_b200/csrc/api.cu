@@ -323,8 +323,8 @@ struct drb_cdae {
 };
 
 // N of the backward GEMMs: hidden plus the constant-one feature that folds db' = colsum(dz) into dW'^T, rounded to 16.
-// tcgen05 tiles are at most 256 wide: for hidden in 241..256 the feature does not fit and the loss kernel accumulates
-// db' itself (cdae_colsum_in_loss).
+// tcgen05 tiles are at most 256 wide: for hidden = 256 the feature does not fit and the loss kernel accumulates db'
+// itself (cdae_colsum_in_loss); for hidden in 241..255 it is the last column of a 256-wide tile.
 static bool cdae_colsum_in_loss(int hidden) { return drb_round_up(hidden + 1, 16) > 256 && hidden <= 256; }
 static int cdae_n2(int hidden) { return (int)drb_round_up(hidden + (cdae_colsum_in_loss(hidden) ? 0 : 1), 16); }
 

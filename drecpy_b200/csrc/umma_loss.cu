@@ -46,7 +46,7 @@ struct LossParams {
   const float* label_count; const uint32_t* label_bits; int words_per_row;
   int loss_kind; float inv_count; int batch;
   float* loss_part;                        // [gridDim.x]
-  float* colsum;                           // NULL, or [N]: db' += column sums of dz (hidden = 241..256: no room for the ones feature)
+  float* colsum;                           // NULL, or [N]: db' += column sums of dz (hidden = 256: no room for the ones feature)
   int m_tiles, n_tiles, row_tiles;         // item tiles (128), batch tiles (BN), 128-row tiles of the dz layout
   DzHalf dzh;                              // H: fp16 dz copies (kernels.h), values scaled by DRB_DZ_F16_SCALE / inv_count
   float out_scale; const float* out_scale_dev;   // H: accumulator -> logit (undoes the operand scaling)

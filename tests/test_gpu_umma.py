@@ -33,8 +33,10 @@ def rel(a, b):
 @pytest.mark.parametrize('U,I,K,B,nnz', [(300, 1682, 50, 64, 12000), (500, 777, 200, 300, 20000),
                                          (257, 1000, 130, 128, 9000), (400, 2049, 64, 129, 15000),
                                          (300, 640, 16, 40, 6000),
-                                         # hidden 241..256: no room for the ones feature, db' summed in the loss epilogue
-                                         (300, 900, 256, 200, 9000), (200, 600, 248, 64, 5000)])
+                                         # hidden 256: no room for the ones feature, db' summed in the loss epilogue
+                                         (300, 900, 256, 200, 9000),
+                                         # hidden 248: the ones feature in column 248 of a 256-wide tile
+                                         (200, 600, 248, 64, 5000)])
 @pytest.mark.parametrize('label_mode,loss', [('batch_mean', 'bce'), ('per_user', 'mse')])
 @pytest.mark.parametrize('gemm', ['tcgen05', 'tcgen05_tf32'])
 def test_tcgen05_step_matches_ffma_and_oracle(U, I, K, B, nnz, label_mode, loss, gemm):
