@@ -67,6 +67,25 @@ class DmfStepArgs(C.Structure):
                 ('t', i32 * 2)]
 
 
+class CaserLayout(C.Structure):
+    _fields_ = [('off_e', i64), ('off_p', i64), ('off_w2', i64), ('off_fv', i64), ('off_fh', i64), ('off_fc', i64),
+                ('off_bv', i64), ('off_bh', i64), ('off_bfc', i64), ('off_b2', i64), ('total', i64),
+                ('ld_e', i32), ('ld_x', i32), ('items_pad', i32)]
+
+
+class CaserDesc(C.Structure):
+    _fields_ = [('n_users', i32), ('n_items', i32), ('L', i32), ('T', i32), ('d', i32), ('n_v', i32), ('n_h', i32),
+                ('neg_ratio', i32), ('dropout_rate', f32), ('params', vp), ('adam_m', vp), ('adam_v', vp),
+                ('grads', vp), ('seq', vp), ('seq_indptr', vp), ('win_off', vp), ('n_windows', i64),
+                ('seen_indptr', vp), ('seen_indices', vp), ('workspace', vp), ('workspace_bytes', i64),
+                ('max_batch', i32)]
+
+
+class CaserStepArgs(C.Structure):
+    _fields_ = [('learning_rate', f32), ('beta1', f32), ('beta2', f32), ('epsilon', f32), ('reg_rate', f32),
+                ('t', i32), ('philox_seed', u64), ('philox_step', u64)]
+
+
 P = C.POINTER
 
 # name -> (restype, argtypes); every symbol include/drb.h declares
@@ -142,6 +161,19 @@ SIGNATURES = {
     'drb_dmf_invalidate_cache': (C.c_int, [vp]),
     'drb_dmf_topk_scratch_bytes': (i64, [vp, i32]),
     'drb_dmf_topk': (C.c_int, [vp, vp, i32, i32, i32, vp, i64, vp, vp, vp]),
+    'drb_caser_layout': (C.c_int, [i32, i32, i32, i32, i32, i32, i32, P(CaserLayout)]),
+    'drb_caser_workspace_bytes': (i64, [i32, i32, i32, i32, i32, i32, i32, i32, i32]),
+    'drb_caser_create': (C.c_int, [vp, P(CaserDesc), P(vp)]),
+    'drb_caser_destroy': (C.c_int, [vp]),
+    'drb_caser_set_optimizer': (C.c_int, [vp, P(OptimDesc)]),
+    'drb_caser_step': (C.c_int, [vp, i32, P(CaserStepArgs), vp]),
+    'drb_caser_loss_buffer': (C.c_int, [vp, P(vp)]),
+    'drb_caser_batch_buffer': (C.c_int, [vp, P(vp), P(vp), P(i32)]),
+    'drb_caser_user_rep': (C.c_int, [vp, vp, i32, vp]),
+    'drb_caser_predict_all': (C.c_int, [vp, vp, i32, vp]),
+    'drb_caser_predict_pairs': (C.c_int, [vp, vp, i32, vp, vp, vp, i32, vp]),
+    'drb_caser_rank_candidates': (C.c_int, [vp, vp, i32, vp, vp, i32, i32, vp, vp, vp]),
+    'drb_caser_topk': (C.c_int, [vp, vp, i32, i32, i32, vp, vp, vp]),
     'drb_debug_cdae_capture_logits': (C.c_int, [vp, vp]),
     'drb_debug_split_tf32': (C.c_int, [vp, vp, i32, i32, i32, vp, vp, vp, vp, i32, i32]),
     'drb_debug_umma_gemm': (C.c_int, [vp, vp, vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp, i32, i32, vp, i32]),

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libdrb.so')
-SOURCES = ['api.cu', 'sparse.cu', 'gemm.cu', 'umma.cu', 'umma_loss.cu', 'umma_score.cu', 'sampled.cu', 'mt_device.cu', 'optim.cu', 'dmf.cu', 'score.cu', 'dmf_topk.cu', 'eval_topk.cu', 'predict.cu', 'host_rng.cpp', 'mt_jump.cpp']
+SOURCES = ['api.cu', 'sparse.cu', 'gemm.cu', 'umma.cu', 'umma_loss.cu', 'umma_score.cu', 'sampled.cu', 'mt_device.cu', 'optim.cu', 'dmf.cu', 'caser.cu', 'score.cu', 'dmf_topk.cu', 'eval_topk.cu', 'predict.cu', 'host_rng.cpp', 'mt_jump.cpp']
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC',
          '-I', os.path.join(ROOT, 'include'), '-I', CSRC]

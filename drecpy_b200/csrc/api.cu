@@ -1856,3 +1856,349 @@ int drb_dmf_invalidate_cache(drb_dmf* m) {
 }
 
 }  // extern "C"
+
+// ========================================================================================== Caser
+struct drb_caser {
+  drb_ctx* ctx;
+  drb_caser_desc d;
+  drb_caser_layout_t L;
+  CaserArgs base;              // sizes, offsets and device arrays of every launch; per-step fields are set per call
+  float *urep, *scores, *loss_part, *reg_part, *loss_scalar, *eye;
+  int32_t *ex_user, *ex_items, *flag;
+  int n_loss_blocks;
+  // the whole step replayed as one graph, with the step size and the philox step at step_scalars
+  StepGraphs graphs;
+  float* step_scalars;
+  drb_optim_desc opt;
+  bool opt_set;
+};
+
+// users per launch of the rank path: a one-hot user representation of this width carries the exact scores (below)
+static constexpr int kCaserRankUsers = 32;
+
+static int caser_fill_layout(int32_t n_users, int32_t n_items, int32_t L, int32_t T, int32_t d, int32_t n_v, int32_t n_h,
+                             drb_caser_layout_t* o) {
+  if (!o) return drb_fail(DRB_E_INVALID, "drb_caser_layout: NULL argument");
+  if (n_users <= 0 || n_items <= 0) return drb_fail(DRB_E_INVALID, "drb_caser_layout: n_users, n_items must be > 0");
+  if (L < 1 || L > 16) return drb_fail(DRB_E_INVALID, "Caser: L must be in [1, 16] (got %d)", L);
+  if (T < 1 || T > 32) return drb_fail(DRB_E_INVALID, "Caser: T must be in [1, 32] (got %d)", T);
+  if (d < 1 || d > 256) return drb_fail(DRB_E_INVALID, "Caser: d must be in [1, 256] (got %d)", d);
+  if (n_v < 1 || n_v > 64) return drb_fail(DRB_E_INVALID, "Caser: n_v must be in [1, 64] (got %d)", n_v);
+  if (n_h < 1 || n_h > 64) return drb_fail(DRB_E_INVALID, "Caser: n_h must be in [1, 64] (got %d)", n_h);
+  std::memset(o, 0, sizeof(*o));
+  o->ld_e = (int32_t)drb_round_up(d, 4);
+  o->ld_x = (int32_t)drb_round_up(2 * d, 4);
+  o->items_pad = (int32_t)drb_round_up(n_items, 4);
+  const int64_t F = (int64_t)n_v * d + (int64_t)n_h * L;
+  int64_t off = 0;
+  auto take = [&](int64_t n) { const int64_t r = off; off += drb_round_up(n, 4); return r; };
+  o->off_e = take((int64_t)n_items * o->ld_e);
+  o->off_p = take((int64_t)n_users * o->ld_e);
+  o->off_w2 = take((int64_t)n_items * o->ld_x);
+  o->off_fv = take((int64_t)L * n_v);
+  o->off_fh = take((int64_t)n_h * d * L * (L + 1) / 2);
+  o->off_fc = take(F * d);
+  o->off_bv = take(n_v);
+  o->off_bh = take((int64_t)L * n_h);
+  o->off_bfc = take(d);
+  o->off_b2 = take(n_items);
+  o->total = off;
+  return DRB_OK;
+}
+
+static CaserArgs caser_args(const drb_caser_layout_t& Lo, int n_users, int n_items, int L, int T, int d, int n_v, int n_h,
+                            int neg_ratio) {
+  CaserArgs a{};
+  a.n_users = n_users; a.n_items = n_items; a.L = L; a.T = T; a.d = d; a.n_v = n_v; a.n_h = n_h;
+  a.n_tgt = T * (1 + neg_ratio);
+  a.F = n_v * d + n_h * L; a.n_fh = n_h * d * L * (L + 1) / 2; a.n_conv = n_h * L * (L + 1) / 2;
+  a.lde = Lo.ld_e; a.ldx = Lo.ld_x;
+  a.off_e = Lo.off_e; a.off_p = Lo.off_p; a.off_w2 = Lo.off_w2; a.off_fv = Lo.off_fv; a.off_fh = Lo.off_fh;
+  a.off_fc = Lo.off_fc; a.off_bv = Lo.off_bv; a.off_bh = Lo.off_bh; a.off_bfc = Lo.off_bfc; a.off_b2 = Lo.off_b2;
+  return a;
+}
+
+static int64_t caser_carve(drb_caser* m, void* base, const drb_caser_layout_t& Lo, int n_items, int row, int max_batch) {
+  Carver c(base);
+  const int64_t B = max_batch;
+  float* urep = c.take<float>(B * Lo.ld_x);
+  float* scores = c.take<float>(B * Lo.items_pad);
+  float* lp = c.take<float>(1024);
+  float* rp = c.take<float>(256 * 16);
+  float* ls = c.take<float>(64);
+  float* eye = c.take<float>(kCaserRankUsers * kCaserRankUsers);
+  int32_t* eu = c.take<int32_t>(B);
+  int32_t* ei = c.take<int32_t>(B * row);
+  int32_t* flag = c.take<int32_t>(4);
+  if (m) {
+    m->urep = urep; m->scores = scores; m->loss_part = lp; m->reg_part = rp; m->loss_scalar = ls; m->eye = eye;
+    m->ex_user = eu; m->ex_items = ei; m->flag = flag;
+    m->step_scalars = ls + 16;
+  }
+  (void)n_items;
+  return c.off;
+}
+
+static int caser_check_sizes(const drb_caser_layout_t& Lo, int L, int T, int d, int n_v, int n_h, int neg_ratio) {
+  if (neg_ratio < 0 || neg_ratio > 1000) return drb_fail(DRB_E_INVALID, "Caser: neg_ratio must be in [0, 1000] (got %d)", neg_ratio);
+  const CaserArgs a = caser_args(Lo, 1, 1, L, T, d, n_v, n_h, neg_ratio);
+  const int64_t smem = caser_smem_bytes(a, true);
+  if (smem > kCaserMaxSmem)
+    return drb_fail(DRB_E_INVALID, "Caser: L=%d, T=%d, d=%d, n_v=%d, n_h=%d, neg_ratio=%d need %lld bytes of shared memory "
+                    "per CTA for the conv / fc weights and their gradients (at most %lld)", L, T, d, n_v, n_h, neg_ratio,
+                    (long long)smem, (long long)kCaserMaxSmem);
+  return DRB_OK;
+}
+
+extern "C" {
+
+int drb_caser_layout(int32_t n_users, int32_t n_items, int32_t L, int32_t T, int32_t d, int32_t n_v, int32_t n_h,
+                     drb_caser_layout_t* out) {
+  int r = caser_fill_layout(n_users, n_items, L, T, d, n_v, n_h, out);
+  if (r) return r;
+  return caser_check_sizes(*out, L, T, d, n_v, n_h, 0);
+}
+
+int64_t drb_caser_workspace_bytes(int32_t n_users, int32_t n_items, int32_t L, int32_t T, int32_t d, int32_t n_v,
+                                  int32_t n_h, int32_t neg_ratio, int32_t max_batch) {
+  drb_caser_layout_t Lo;
+  if (drb_caser_layout(n_users, n_items, L, T, d, n_v, n_h, &Lo) || max_batch <= 0 || neg_ratio < 0) return -1;
+  return caser_carve(nullptr, nullptr, Lo, n_items, L + T * (1 + neg_ratio), max_batch);
+}
+
+int drb_caser_create(drb_ctx* ctx, const drb_caser_desc* d, drb_caser** out) {
+  if (!ctx || !d || !out) return drb_fail(DRB_E_INVALID, "drb_caser_create: NULL argument");
+  drb_caser_layout_t Lo;
+  int r = drb_caser_layout(d->n_users, d->n_items, d->L, d->T, d->d, d->n_v, d->n_h, &Lo);
+  if (r) return r;
+  if ((r = caser_check_sizes(Lo, d->L, d->T, d->d, d->n_v, d->n_h, d->neg_ratio))) return r;
+  if (!(d->dropout_rate >= 0.f && d->dropout_rate < 1.f))
+    return drb_fail(DRB_E_INVALID, "drb_caser_create: dropout_rate must be in [0, 1)");
+  if (!d->params || !d->seq || !d->seq_indptr || !d->win_off || !d->seen_indptr || !d->seen_indices || !d->workspace ||
+      d->max_batch <= 0)
+    return drb_fail(DRB_E_INVALID, "drb_caser_create: params, sequences, windows, stored rows and workspace are required");
+  if (((uintptr_t)d->params | (uintptr_t)d->adam_m | (uintptr_t)d->adam_v | (uintptr_t)d->grads |
+       (uintptr_t)d->workspace) & 15)
+    return drb_fail(DRB_E_INVALID, "drb_caser_create: arenas and workspace must be 16-byte aligned");
+  drb_caser* m = new (std::nothrow) drb_caser();
+  if (!m) return drb_fail(DRB_E_NOMEM, "out of memory");
+  m->ctx = ctx; m->d = *d; m->L = Lo;
+  const int row = d->L + d->T * (1 + d->neg_ratio);
+  const int64_t need = caser_carve(m, d->workspace, Lo, d->n_items, row, d->max_batch);
+  if (need > d->workspace_bytes) {
+    delete m;
+    return drb_fail(DRB_E_INVALID, "drb_caser_create: workspace too small (%lld < %lld bytes)",
+                    (long long)d->workspace_bytes, (long long)need);
+  }
+  CaserArgs& a = m->base;
+  a = caser_args(Lo, d->n_users, d->n_items, d->L, d->T, d->d, d->n_v, d->n_h, d->neg_ratio);
+  a.params = d->params; a.grads = d->grads;
+  a.seq = d->seq; a.seq_off = d->seq_indptr; a.win_off = d->win_off; a.n_windows = d->n_windows;
+  a.seen_indptr = d->seen_indptr; a.seen_indices = d->seen_indices;
+  a.ex_user = m->ex_user; a.ex_items = m->ex_items;
+  a.dropout = d->dropout_rate; a.keep_scale = 1.0f / (1.0f - d->dropout_rate);
+  a.loss_part = m->loss_part;
+  float eye[kCaserRankUsers * kCaserRankUsers] = {};
+  for (int i = 0; i < kCaserRankUsers; i++) eye[i * kCaserRankUsers + i] = 1.f;
+  if (cudaMemsetAsync(m->loss_scalar, 0, 64 * sizeof(float), ctx->stream) != cudaSuccess ||
+      cudaMemcpyAsync(m->eye, eye, sizeof(eye), cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess ||
+      cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+    delete m;
+    return drb_fail(DRB_E_CUDA, "drb_caser_create: workspace initialisation failed");
+  }
+  *out = m;
+  return DRB_OK;
+}
+
+int drb_caser_destroy(drb_caser* m) {
+  delete m;
+  return DRB_OK;
+}
+
+int drb_caser_set_optimizer(drb_caser* m, const drb_optim_desc* opt) {
+  if (!m) return drb_fail(DRB_E_INVALID, "drb_caser_set_optimizer: NULL model");
+  int r = optim_check(opt, "drb_caser_set_optimizer");
+  if (r) return r;
+  m->opt = *opt;
+  m->opt_set = true;
+  m->graphs.clear();
+  return DRB_OK;
+}
+
+}  // extern "C"
+
+// one step on ctx->stream; scal_dev != NULL: the step size and the philox step come from device memory (graph capture)
+static int caser_step_body(drb_caser* m, int32_t batch, const drb_caser_step_args* s, float* loss_out, float* scal_dev) {
+  drb_ctx* ctx = m->ctx;
+  int r;
+  DRB_CUDA_TRY(ctx, cudaMemsetAsync(m->d.grads, 0, (size_t)m->L.total * sizeof(float), ctx->stream));
+  CaserArgs a = m->base;
+  a.seed = s->philox_seed; a.step = s->philox_step;
+  a.step_dev = scal_dev ? reinterpret_cast<const uint32_t*>(scal_dev + 1) : nullptr;
+  a.inv_count = 1.0f / (float)((int64_t)batch * a.n_tgt);
+  if ((r = launch_caser_sample(ctx, a, batch))) return r;
+  int n_blocks = 0;
+  if ((r = launch_caser_step(ctx, a, batch, &n_blocks))) return r;
+  AdamArgs ad{};
+  ad.w = m->d.params; ad.m = m->d.adam_m; ad.v = m->d.adam_v; ad.g = m->d.grads;
+  const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, s->beta1, s->beta2, s->epsilon);
+  OptimExtra ox;
+  optim_fill_args(opt, ad, ox);
+  ad.alpha_dev = scal_dev;
+  const float alpha = drb_optim_step_size(opt, s->learning_rate, s->t);
+  ad.seg[0] = AdamSeg{0, m->L.off_bv / 4, alpha, 2.0f * s->reg_rate, s->reg_rate, 0};   // tensors under L2
+  ad.seg[1] = AdamSeg{m->L.off_bv / 4, (m->L.total - m->L.off_bv) / 4, alpha, 0.f, 0.f, 0};
+  ad.nseg = 2;
+  ad.reg_part = m->reg_part;
+  ad.fin_loss_part = m->loss_part; ad.fin_n_loss = n_blocks; ad.fin_scale = a.inv_count;
+  ad.fin_n_reg = 0; ad.fin_reg_part = nullptr; ad.fin_loss_out = loss_out;
+  ad.fin_ticket = reinterpret_cast<unsigned int*>(m->loss_scalar + 48);
+  int n_reg = 0;
+  return launch_adam(ctx, ad, &n_reg, ox);
+}
+
+extern "C" {
+
+int drb_caser_step(drb_caser* m, int32_t batch, const drb_caser_step_args* s, float* loss_out) {
+  if (!m || !s || !loss_out) return drb_fail(DRB_E_INVALID, "drb_caser_step: NULL argument");
+  if (batch <= 0 || batch > m->d.max_batch)
+    return drb_fail(DRB_E_INVALID, "drb_caser_step: batch %d outside (0, max_batch=%d]", batch, m->d.max_batch);
+  if (!m->d.adam_m || !m->d.adam_v || !m->d.grads)
+    return drb_fail(DRB_E_STATE, "drb_caser_step: model was created without optimizer arenas");
+  if (m->d.n_windows <= 0) return drb_fail(DRB_E_STATE, "drb_caser_step: no user has L + T items");
+  drb_ctx* ctx = m->ctx;
+  if (ctx->sticky) return drb_fail(DRB_E_CUDA, "context has a sticky CUDA error (%d)", ctx->sticky);
+  if (m->graphs.off || ctx->profile) return caser_step_body(m, batch, s, loss_out, nullptr);
+  const StepGraphKey key{loss_out, batch, 0, 0, 0, s->beta1, s->beta2, s->epsilon, s->reg_rate, s->philox_seed};
+  const StepGraphs::Entry* g = m->graphs.get(ctx, key, [&] { return caser_step_body(m, batch, s, loss_out, m->step_scalars); });
+  if (!g) return caser_step_body(m, batch, s, loss_out, nullptr);
+  const drb_optim_desc opt = effective_optim(m->opt_set, m->opt, s->beta1, s->beta2, s->epsilon);
+  float vals[3];
+  vals[0] = drb_optim_step_size(opt, s->learning_rate, s->t);
+  const uint32_t slo = (uint32_t)s->philox_step, shi = (uint32_t)(s->philox_step >> 32);
+  std::memcpy(&vals[1], &slo, 4);
+  std::memcpy(&vals[2], &shi, 4);
+  return m->graphs.replay(ctx, g, m->step_scalars, vals, 3);
+}
+
+int drb_caser_loss_buffer(drb_caser* m, float** ptr) {
+  if (!m || !ptr) return drb_fail(DRB_E_INVALID, "drb_caser_loss_buffer: NULL argument");
+  *ptr = m->loss_scalar;
+  return DRB_OK;
+}
+
+int drb_caser_batch_buffer(drb_caser* m, int32_t** users, int32_t** items, int32_t* row_len) {
+  if (!m || !users || !items || !row_len) return drb_fail(DRB_E_INVALID, "drb_caser_batch_buffer: NULL argument");
+  *users = m->ex_user; *items = m->ex_items; *row_len = m->base.L + m->base.n_tgt;
+  return DRB_OK;
+}
+
+int drb_caser_user_rep(drb_caser* m, const int32_t* uids, int32_t n, float* x_out) {
+  if (!m || !uids || !x_out || n < 0 || n > m->d.max_batch) return drb_fail(DRB_E_INVALID, "drb_caser_user_rep: bad argument");
+  return launch_caser_user_rep(m->ctx, m->base, uids, n, x_out);
+}
+
+}  // extern "C"
+
+// sigmoid(x W2^T + b2) for c <= max_batch users into out [c][items_pad]: the fmaf chain every Caser score comes from
+static int caser_scores_chunk(drb_caser* m, const int32_t* uids, int c, float* out) {
+  int r = launch_caser_user_rep(m->ctx, m->base, uids, c, m->urep);
+  if (r) return r;
+  GemmArgs g{};
+  g.A = m->urep; g.lda = m->L.ld_x; g.B = m->d.params + m->L.off_w2; g.ldb = m->L.ld_x; g.C = out;
+  g.ldc = m->L.items_pad; g.M = c; g.N = m->d.n_items; g.Kred = m->L.ld_x; g.splits = 1;
+  g.bias = m->d.params + m->L.off_b2; g.act = DRB_ACT_SIGMOID;
+  return launch_gemm(m->ctx, LAYOUT_KK, EPI_BIAS_ACT, g);
+}
+
+extern "C" {
+
+int drb_caser_predict_all(drb_caser* m, const int32_t* uids, int32_t n, float* out) {
+  if (!m || !uids || !out || n < 0) return drb_fail(DRB_E_INVALID, "drb_caser_predict_all: bad argument");
+  for (int32_t o = 0; o < n; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, n - o);
+    int r = caser_scores_chunk(m, uids + o, c, out + (int64_t)o * m->L.items_pad);
+    if (r) return r;
+  }
+  return DRB_OK;
+}
+
+int drb_caser_predict_pairs(drb_caser* m, const int32_t* users, int32_t n_users, const int64_t* pair_off,
+                            const int32_t* pair_iid, const int32_t* pair_dst, int32_t n, float* out) {
+  if (!m || (n > 0 && !out)) return drb_fail(DRB_E_INVALID, "drb_caser_predict_pairs: NULL argument");
+  const PairArgs p{users, n_users, pair_off, pair_iid, pair_dst, n};
+  if (n_users == 0 && n == 0) return DRB_OK;
+  int r = pair_args_check(m->ctx, "drb_caser_predict_pairs", p, m->d.n_users, m->d.n_items, m->flag);
+  if (r) return r;
+  for (int32_t o = 0; o < n_users; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, n_users - o);
+    if ((r = launch_caser_user_rep(m->ctx, m->base, users + o, c, m->urep))) return r;
+    if ((r = launch_cdae_pair_scores(m->ctx, p, o, c, m->urep, m->d.params + m->L.off_w2, m->d.params + m->L.off_b2,
+                                     m->L.ld_x, out)))
+      return r;
+  }
+  return DRB_OK;
+}
+
+// The rank path takes its scores from the chain of drb_caser_predict_all: for a block of 32 users the GEMM forms the
+// logits x W2^T transposed ([n_items][32], no bias), and k_rank_candidates scores candidate j of user u as the dot
+// product of that row with the one-hot vector e_u (1 * logit plus zeros: exactly the logit), plus b2[j], through the
+// same sigmoid.  Catalog-long candidate lists sort their keys in the score buffer.
+int drb_caser_rank_candidates(drb_caser* m, const int32_t* uids, int32_t n, const int32_t* cand,
+                              const int32_t* cand_count, int32_t max_cand, int32_t novelty, int32_t* out_iid,
+                              float* out_score, int32_t* n_out) {
+  if (!m || !uids || !cand || !cand_count || !out_iid || !out_score || !n_out || n < 0 || max_cand < 1)
+    return drb_fail(DRB_E_INVALID, "drb_caser_rank_candidates: bad argument");
+  const int U = kCaserRankUsers;
+  const int64_t logit_floats = (int64_t)m->d.n_items * U;
+  if (m->d.max_batch < U || logit_floats > (int64_t)m->d.max_batch * m->L.items_pad)
+    return drb_fail(DRB_E_INVALID, "drb_caser_rank_candidates: max_batch must be >= %d", U);
+  float* logits = m->scores;
+  void* scratch = m->scores + drb_round_up(logit_floats, 64);
+  const int64_t scratch_bytes = ((int64_t)m->d.max_batch * m->L.items_pad - drb_round_up(logit_floats, 64)) * 4;
+  int64_t per = U;
+  if (max_cand > 4096) {
+    per = std::min<int64_t>(per, rank_scratch_rows(scratch_bytes, max_cand));
+    if (per < 1) return drb_fail(DRB_E_INVALID, "drb_caser_rank_candidates: max_cand %d does not fit the workspace", max_cand);
+  }
+  for (int32_t o = 0; o < n; o += U) {
+    const int c = std::min(U, n - o);
+    int r = launch_caser_user_rep(m->ctx, m->base, uids + o, c, m->urep);
+    if (r) return r;
+    GemmArgs g{};
+    g.A = m->d.params + m->L.off_w2; g.lda = m->L.ld_x; g.B = m->urep; g.ldb = m->L.ld_x; g.C = logits; g.ldc = U;
+    g.M = m->d.n_items; g.N = c; g.Kred = m->L.ld_x; g.splits = 1;
+    if ((r = launch_gemm(m->ctx, LAYOUT_KK, EPI_STORE, g))) return r;
+    for (int q = 0; q < c; q += (int)per) {
+      const int cc = std::min<int>((int)per, c - q);
+      CandScoreArgs a{};
+      a.urep = m->eye + q * U; a.ld_u = U; a.table = logits; a.ld_t = U;
+      a.bias = m->d.params + m->L.off_b2; a.width = U; a.mode = 0;
+      const int64_t u0 = o + q;
+      a.uids = uids + u0; a.cand = cand + u0 * max_cand; a.cand_count = cand_count + u0; a.max_cand = max_cand;
+      a.seen_indptr = m->d.seen_indptr; a.seen_indices = m->d.seen_indices; a.novelty = novelty;
+      a.out_iid = out_iid + u0 * max_cand; a.out_score = out_score + u0 * max_cand; a.n_out = n_out + u0;
+      if ((r = launch_rank_candidates(m->ctx, a, cc, scratch, scratch_bytes))) return r;
+    }
+  }
+  return DRB_OK;
+}
+
+int drb_caser_topk(drb_caser* m, const int32_t* uids, int32_t n, int32_t k, int32_t novelty, int32_t* out_iid,
+                   float* out_score, int32_t* n_out) {
+  if (!m || !uids || !out_iid || !out_score || !n_out || n < 0) return drb_fail(DRB_E_INVALID, "drb_caser_topk: bad argument");
+  if (k < 1 || k > 2048) return drb_fail(DRB_E_INVALID, "drb_caser_topk: k must be in [1, 2048]");
+  for (int32_t o = 0; o < n; o += m->d.max_batch) {
+    const int c = std::min(m->d.max_batch, n - o);
+    int r;
+    if ((r = caser_scores_chunk(m, uids + o, c, m->scores))) return r;
+    TopkArgs t{};
+    t.scores = m->scores; t.ld = m->L.items_pad; t.n_items = m->d.n_items; t.uids = uids + o;
+    t.seen_indptr = m->d.seen_indptr; t.seen_indices = m->d.seen_indices; t.novelty = novelty; t.k = k;
+    t.out_iid = out_iid + (int64_t)o * k; t.out_score = out_score + (int64_t)o * k; t.n_out = n_out + o;
+    if ((r = launch_topk(m->ctx, t, c))) return r;
+  }
+  return DRB_OK;
+}
+
+}  // extern "C"

@@ -328,4 +328,26 @@ int launch_cdae_pair_scores(drb_ctx* ctx, const PairArgs& p, int u0, int c, cons
 int launch_dmf_pair_head(drb_ctx* ctx, const PairArgs& p, int u0, int c, const float* urep, int ld_u,
                          const float* irep, int ld_i, int width, float* out);
 
+// ------------------------------------------------------------------ caser.cu
+// Caser (oracle/caser.py): device batch sampler, fused forward + backward of one step, user representation.
+struct CaserArgs {
+  int n_users, n_items, L, T, d, n_v, n_h, n_tgt;   // n_tgt = T (1 + neg_ratio): targets, then negatives
+  int F, n_fh, n_conv, lde, ldx;                    // F = n_v d + n_h L; n_fh = n_h d L (L + 1) / 2; n_conv = n_h L (L + 1) / 2
+  int64_t off_e, off_p, off_w2, off_fv, off_fh, off_fc, off_bv, off_bh, off_bfc, off_b2;
+  const float* params; float* grads;
+  const int32_t* seq; const int64_t* seq_off;       // per-user sequences (CSR over users)
+  const int64_t* win_off; int64_t n_windows;        // [n_users + 1] prefix sums of the windows of L + T items
+  const int64_t* seen_indptr; const int32_t* seen_indices;   // all stored items per user, sorted
+  int32_t* ex_user; int32_t* ex_items;              // [batch], [batch][L + n_tgt]
+  float dropout, keep_scale, inv_count;
+  uint64_t seed, step; const uint32_t* step_dev;    // step_dev: {lo, hi} in device memory (graph replay)
+  float* loss_part;                                 // [grid] raw sums of the loss terms
+};
+constexpr int64_t kCaserMaxSmem = 227 * 1024;
+int64_t caser_smem_bytes(const CaserArgs& a, bool train);
+int launch_caser_sample(drb_ctx* ctx, const CaserArgs& a, int batch);
+int launch_caser_step(drb_ctx* ctx, const CaserArgs& a, int batch, int* n_blocks_out);
+// out[n][ldx] = [z; P[u]] for users uids[0..n), no dropout
+int launch_caser_user_rep(drb_ctx* ctx, const CaserArgs& a, const int32_t* uids, int n, float* out);
+
 #endif

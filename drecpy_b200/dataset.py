@@ -52,11 +52,13 @@ def _unique_sorted(keys):
 
 
 class InteractionData:
-    def __init__(self, users, items, interactions):
+    def __init__(self, users, items, interactions, timestamp=None):
         self.user = np.asarray(users)
         self.item = np.asarray(items)
         self.interaction = np.asarray(interactions)
         assert len(self.user) == len(self.item) == len(self.interaction)
+        self.timestamp = None if timestamp is None else np.asarray(timestamp)     # optional: orders Caser's sequences
+        assert self.timestamp is None or len(self.timestamp) == len(self.user)
         self.has_internal_ids = False
         self.uid = self.iid = None
         self._users = self._items = None
@@ -65,8 +67,10 @@ class InteractionData:
 
     # ------------------------------------------------------------------ construction
     @classmethod
-    def read_df(cls, df, user_label='user', item_label='item', interaction_label='interaction', **kwds):
-        return cls(df[user_label].values, df[item_label].values, df[interaction_label].values)
+    def read_df(cls, df, user_label='user', item_label='item', interaction_label='interaction', timestamp_label=None,
+                **kwds):
+        ts = df[timestamp_label].values if timestamp_label is not None else None
+        return cls(df[user_label].values, df[item_label].values, df[interaction_label].values, timestamp=ts)
 
     @classmethod
     def from_dataset(cls, ds):
@@ -75,7 +79,8 @@ class InteractionData:
             return ds
         df = getattr(ds, '_df', None)
         if df is not None and all(c in df.columns for c in ('user', 'item', 'interaction')):
-            return cls(df['user'].values, df['item'].values, df['interaction'].values)
+            ts = df['timestamp'].values if 'timestamp' in df.columns else None
+            return cls(df['user'].values, df['item'].values, df['interaction'].values, timestamp=ts)
         if hasattr(ds, 'values_list'):
             rows = ds.values_list(['user', 'item', 'interaction'], to_list=True)
             u, i, v = zip(*rows) if rows else ((), (), ())

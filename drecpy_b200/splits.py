@@ -4,7 +4,8 @@ Mirrors DRecPy/Evaluation/Splits/leave_k_out.py:14-135 -- same signature, assert
 (random.Random(seed + idx + 1): the seed is incremented before each user's generator is created, :68-69) and row
 selection (rng.sample over the user's rows in DataFrame order, :131-133) -- but for all users in one native call
 (drb_leave_k_out, host C++ MT19937 replay, multi-threaded) instead of one `select('user == ...')` scan per user.
-Returns two InteractionData objects whose rows keep the order of the input (InteractionDataset.drop semantics).
+Returns two InteractionData objects whose rows keep the order of the input (InteractionDataset.drop semantics), with
+the input's timestamps when it has them.
 """
 import os
 from heapq import heappush, heapreplace
@@ -71,5 +72,6 @@ def leave_k_out(interaction_dataset, k=1, min_user_interactions=0, last_timestam
     row_flag = np.empty(len(ds), np.uint8)
     row_flag[order] = flags
     tr, te = np.flatnonzero(row_flag == 0), np.flatnonzero(row_flag == 1)
-    return (InteractionData(ds.user[tr], ds.item[tr], ds.interaction[tr]),
-            InteractionData(ds.user[te], ds.item[te], ds.interaction[te]))
+    ts = ds.timestamp if ds.timestamp is not None else (None if timestamps is None else np.asarray(timestamps))
+    return (InteractionData(ds.user[tr], ds.item[tr], ds.interaction[tr], None if ts is None else ts[tr]),
+            InteractionData(ds.user[te], ds.item[te], ds.interaction[te], None if ts is None else ts[te]))

@@ -48,6 +48,7 @@ typedef struct drb_rng drb_rng;
 typedef struct drb_sampler drb_sampler;
 typedef struct drb_cdae drb_cdae;
 typedef struct drb_dmf drb_dmf;
+typedef struct drb_caser drb_caser;
 
 /* ------------------------------------------------------------------ diagnostics */
 int drb_version(void);
@@ -411,6 +412,84 @@ int drb_dmf_invalidate_cache(drb_dmf* m);
 int64_t drb_dmf_topk_scratch_bytes(drb_dmf* m, int32_t k);
 int drb_dmf_topk(drb_dmf* m, const int32_t* uids, int32_t n, int32_t k, int32_t novelty, void* scratch,
                  int64_t scratch_bytes, int32_t* out_iid, float* out_score, int32_t* n_out);
+
+/* ------------------------------------------------------------------ Caser
+ * Tang & Wang, "Personalized Top-N Sequential Recommendation via Convolutional Sequence Embedding" (WSDM 2018), the
+ * third deep recommender of DRecPy.  The model, its batch sampler and its dropout stream are pinned by oracle/caser.py
+ * (parity with DRecPy's TensorFlow Caser is unpinned, DESIGN.md section 8).  Supported sizes: 1 <= L <= 16,
+ * 1 <= T <= 32, 1 <= d <= 256, 1 <= n_v, n_h <= 64, and the conv / fc weights with their gradients must fit the 227 KB
+ * of shared memory of one CTA (drb_caser_layout fails with a message otherwise).
+ * Arena layout (floats), every tensor 16-byte aligned, first the tensors under L2, then those without:
+ *   [ E n_items x ld_e | P n_users x ld_e | W2 n_items x ld_x | Fv L x n_v | Fh | fc (n_v d + n_h L) x d ]
+ *   [ bv n_v | bh L x n_h | b_fc d | b2 n_items ]
+ * ld_e = d and ld_x = 2d rounded up to a multiple of 4 (pad columns stay zero); Fh holds the horizontal kernels
+ * h = 1 .. L one after the other, kernel h [h][d][n_h] at n_h d (h - 1) h / 2; bh row h - 1 is the bias of kernel h;
+ * fc is Keras-shaped [in][out], its input ordered [vertical output c d + k for c < n_v, k < d; pooled horizontal output
+ * (h - 1) n_h + f].  The L2 tensors end at off_bv. */
+typedef struct {
+  int64_t off_e, off_p, off_w2, off_fv, off_fh, off_fc, off_bv, off_bh, off_bfc, off_b2, total;
+  int32_t ld_e, ld_x, items_pad;
+} drb_caser_layout_t;
+int drb_caser_layout(int32_t n_users, int32_t n_items, int32_t L, int32_t T, int32_t d, int32_t n_v, int32_t n_h,
+                     drb_caser_layout_t* out);
+int64_t drb_caser_workspace_bytes(int32_t n_users, int32_t n_items, int32_t L, int32_t T, int32_t d, int32_t n_v,
+                                  int32_t n_h, int32_t neg_ratio, int32_t max_batch);
+
+typedef struct {
+  int32_t n_users, n_items, L, T, d, n_v, n_h, neg_ratio;
+  float dropout_rate;          /* in [0, 1) */
+  float* params;               /* device arenas (caller-owned) */
+  float* adam_m;
+  float* adam_v;
+  float* grads;
+  /* device: the training sequences (CSR over users, each user's items in sequence order) and the prefix sums of the
+   * windows of L + T consecutive items per user ([n_users + 1], win_off[n_users] = n_windows > 0) */
+  const int32_t* seq; const int64_t* seq_indptr;
+  const int64_t* win_off; int64_t n_windows;
+  const int64_t* seen_indptr;  /* device CSR of ALL stored rows, column-sorted: negatives and the novelty filter */
+  const int32_t* seen_indices;
+  void* workspace;             /* device, >= drb_caser_workspace_bytes(...) */
+  int64_t workspace_bytes;
+  int32_t max_batch;           /* windows per step and users per scoring chunk */
+} drb_caser_desc;
+
+typedef struct {
+  float learning_rate, beta1, beta2, epsilon;
+  float reg_rate;
+  int32_t t;                   /* optimizer step counter, the same for every tensor */
+  uint64_t philox_seed;        /* key of the sampler and dropout streams */
+  uint64_t philox_step;        /* counter words 2-3 of every draw of this step */
+} drb_caser_step_args;
+
+int drb_caser_create(drb_ctx* ctx, const drb_caser_desc* desc, drb_caser** out);
+int drb_caser_destroy(drb_caser* m);
+/* drb_cdae_set_optimizer for Caser */
+int drb_caser_set_optimizer(drb_caser* m, const drb_optim_desc* opt);
+/* One training step of `batch` windows, drawn on the device (nothing is read from the host): sampler, fused forward +
+ * backward into the gradient arena (raw gradients, without the L2 term), the dense update of the whole arena, and the
+ * loss.  loss_out: device float[2] ([0] reported loss = mean BCE + reg_rate sum w^2 over the L2 tensors, [1] the BCE
+ * term).  Launch-bound shapes replay the step as one CUDA graph. */
+int drb_caser_step(drb_caser* m, int32_t batch, const drb_caser_step_args* args, float* loss_out);
+int drb_caser_loss_buffer(drb_caser* m, float** ptr);   /* device float[2] for loss_out */
+/* The batch of the last step (device): users[max_batch], items[max_batch][row_len] = L inputs, T targets,
+ * T * neg_ratio negatives. */
+int drb_caser_batch_buffer(drb_caser* m, int32_t** users, int32_t** items, int32_t* row_len);
+/* x[n][ld_x] = [z; P[u]] for n users (device), from the last L items of each sequence, left-padded with zero rows,
+ * without dropout.  n <= max_batch. */
+int drb_caser_user_rep(drb_caser* m, const int32_t* uids, int32_t n, float* x_out);
+/* Scores sigmoid(x W2[j] + b2[j]) of n users over all items: out[n x items_pad] (one fmaf chain over ld_x). */
+int drb_caser_predict_all(drb_caser* m, const int32_t* uids, int32_t n, float* out);
+/* Pair scores with the arguments of drb_cdae_predict_pairs; bit for bit the elements of drb_caser_predict_all. */
+int drb_caser_predict_pairs(drb_caser* m, const int32_t* users, int32_t n_users, const int64_t* pair_off,
+                            const int32_t* pair_iid, const int32_t* pair_dst, int32_t n, float* out);
+/* Contract of drb_cdae_rank_candidates; every score is bit for bit the drb_caser_predict_all element. */
+int drb_caser_rank_candidates(drb_caser* m, const int32_t* uids, int32_t n, const int32_t* cand,
+                              const int32_t* cand_count, int32_t max_cand, int32_t novelty,
+                              int32_t* out_iid, float* out_score, int32_t* n_out);
+/* Full-catalog top-k, contract of drb_cdae_topk_exact (1 <= k <= 2048); scores bit for bit those of
+ * drb_caser_predict_all. */
+int drb_caser_topk(drb_caser* m, const int32_t* uids, int32_t n, int32_t k, int32_t novelty,
+                   int32_t* out_iid, float* out_score, int32_t* n_out);
 
 /* ------------------------------------------------------------------ kernel-level test hooks (tests/ only)
  * The tcgen05 GEMM building blocks of the CDAE step, exposed so that tests can check them in isolation against
